@@ -1,7 +1,7 @@
 """bench.py -- the BASELINE.json configurations of the fusion / co-attention hot path on N B200s of one node.
 
     python bench.py [--config c1|c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--batch B] [--precision bf16|fp32]
+                    [--batch B] [--precision bf16|fp32] [--dump-outputs DIR]
 
 Configurations (BASELINE.json `configs`, SURVEY.md 8d "Config -> concrete run"); the default, and the one the metric is
 quoted on, is c2:
@@ -18,6 +18,15 @@ Prints ONE JSON line (rank 0).  `value` = whole-job samples/s with inputs reside
 the public module API with HOST (pinned) inputs, H2D copies and a D2H read of the result inside the timed region;
 `roofline` = the configuration's dominant kernel timed live with CUDA events; `cpu_baseline` = the oracle port of the
 reference's algorithm on the host cores (bounded sample).  `--impl reference` times that CPU path alone (rank 0 only).
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller on rank 0 as DIR/<name>.npy (float32):
+for c1..c4 the loss of rank 0's batch, for c5 the log-probabilities of rank 0's rows of the largest batch.  Inputs,
+weights and dropout seeds depend on the arguments only, so two builds run with the same arguments can be compared array
+by array.  The parameters are not dumped: they carry every step before the last, and Adam turns the rounding noise of
+the atomic gradient sums into whole +-lr steps wherever a gradient is near zero, so they differ from run to run by far
+more than rounding (tools/dump_repro.py measures both).
+
+The tree may be read-only: scratch files (the feature shard, the clock samples) go to the temporary directory.
 """
 from __future__ import annotations
 
@@ -27,6 +36,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 import types
 
@@ -89,6 +99,28 @@ def measured_peaks():
     return {"bf16_sustained": 1400.0, "bf16_burst": 1590.0, "hbm": 6650.0, "source": "fallback"}
 
 
+DUMP_BYTES = 60 << 20        # payload of all --dump-outputs arrays together; the .npy headers fit in the rest of 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of `arrays` (name -> tensor) as <out_dir>/<name>.npy in float32.  A tensor larger than its equal
+    share of DUMP_BYTES is written as a sample of its flattened elements, at positions drawn from a fixed seed (the same
+    positions in every run)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float()
+        how = "shape %s" % (list(a.shape),)
+        if a.numel() > share:
+            pos = np.sort(np.random.default_rng(0).choice(a.numel(), share, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(pos).to(a.device)]
+            how += ", seeded sample of %d elements" % share
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+        print("bench: dumped %s (%s)" % (name, how), file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------------------
 # synthetic data (SURVEY.md 8d)
 # ------------------------------------------------------------------------------------------------
@@ -135,7 +167,7 @@ class ClockSampler:
     def __init__(self, gpu_index=0):
         self.gpu = str(gpu_index)
         self.proc = None
-        self.path = "/tmp/vqa_b200_clocks_%d.csv" % os.getpid()
+        self.path = os.path.join(tempfile.gettempdir(), "vqa_b200_clocks_%d.csv" % os.getpid())
         self.t0 = self.t1 = None
 
     def start(self):
@@ -459,7 +491,7 @@ def run_train(args, wl):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(K):
-            train_step(i % 2)
+            loss = train_step(i % 2)
         e1.record()
         host_enqueue_ms = (time.perf_counter() - h0) * 1e3 / K      # host time to ENQUEUE a step (no sync inside)
         barrier()
@@ -470,13 +502,15 @@ def run_train(args, wl):
             l2_flush.fill_(i & 0xFF)                                  # 256 MB write: evicts the 126 MB L2 (untimed)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            train_step(i % 2)
+            loss = train_step(i % 2)
             b.record()
             evs.append((a, b))
         host_enqueue_ms = (time.perf_counter() - h0) * 1e3 / K
         barrier()
         ms_total = sum(a.elapsed_time(b) for a, b in evs)
     sampler.end()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss})
     if graphed is not None:
         launches = graphed.launches * K
         ktimes = graphed.kernel_times()
@@ -581,7 +615,7 @@ def run_train(args, wl):
     if args.precision == "bf16":
         soft = wl["target"] == "soft"
         shm, shard_path, reader = None, None, None
-        for cand in ("/dev/shm", "/tmp", ROOT):               # a small /dev/shm (container default 64 MB) must not end the run
+        for cand in ("/dev/shm", tempfile.gettempdir()):      # a small /dev/shm (container default 64 MB) must not end the run
             if not (os.path.isdir(cand) and os.access(cand, os.W_OK)):
                 continue
             shard_path = os.path.join(cand, "vqa_b200_bench_%d_%d.shard" % (os.getpid(), rank))
@@ -841,6 +875,8 @@ def run_infer(args, wl):
             ms_dev = sum(a.elapsed_time(b_) for a, b_ in evs) / K
         if rank == 0 and gb == sizes[-1]:
             sampler.end()
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {"out": g.out})
         if n > 0:
             # `e2e`: pinned host inputs -> H2D -> replay -> argmax -> D2H of the predicted answers, every step
             pred_host = torch.zeros(n, dtype=torch.int64).pin_memory()
@@ -984,7 +1020,13 @@ def main():
     ap.add_argument("--graph", type=int, default=1, help="1: capture the train iteration in CUDA graphs (default); 0: eager")
     ap.add_argument("--optimizer", default="fused", choices=["fused", "torch"],
                     help="fused: this repo's multi-tensor Adam (also refreshes the bf16 weight copies); torch: stock")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     wl = WORKLOADS[args.config]
     if args.batch <= 0:
         args.batch = wl["batch"]

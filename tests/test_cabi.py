@@ -47,9 +47,11 @@ def test_release_library_has_no_global_state_hooks():
 
 def test_no_cpu_fallback():
     """The product path must fail loudly on CPU tensors instead of computing something else."""
-    from vqa_attention_networks_b200 import ops
+    from vqa_attention_networks_b200 import Attention_layer, ops
     with pytest.raises(RuntimeError, match="CUDA tensors only"):
         ops.pack_bf16(torch.zeros(4, 8))
+    with pytest.raises(RuntimeError, match="CUDA tensors only"):
+        Attention_layer(16, 1)(torch.zeros(2, 6, 16), torch.zeros(2, 5, 16))
 
 
 def _cfg(**kw):

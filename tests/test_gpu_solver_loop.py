@@ -2,8 +2,8 @@
 package's modules on the B200 -- the train loop and val loop of solver.py:68-153 (stock torch.optim.Adam, KLDivLoss /
 CrossEntropyLoss, `q_l` passed positionally), the checkpoint round trip of solver.py:185-192, a network assembled the way
 networks.py:30-69 assembles AttentionNet, and replicas running concurrently in Python threads on one GPU as
-nn.DataParallel runs them (solver.py:34-36).  The CPU half (tests/test_reference_callers.py) runs the reference's real
-Solver / AttentionNet / clean_state_dict against these classes in the build container."""
+nn.DataParallel runs them (solver.py:34-36).  The reference's state-dict layouts, recorded from the real modules in
+tests/golden/, are checked on the CPU side (tests/test_cabi.py)."""
 import threading
 import types
 
@@ -97,7 +97,7 @@ def test_solver_shaped_train_and_val_loop(name):
 class _AttentionNetLike(nn.Module):
     """The assembly of networks.py:30-69 (img_emb, que_emb, att_num Attention_layers applied alternately to (img, que)
     and (que, img), always-on functional dropout, dim-0 cat + view head, BatchNorm) restated over this package's
-    Attention_layer; the reference class itself is exercised on the CPU side (test_reference_callers.py)."""
+    Attention_layer, whose layout tests/test_cabi.py checks against the reference's (golden data)."""
 
     def __init__(self, block_num, word_num, img_size, vocab_size, embed_size, att_num, output_size):
         super().__init__()
