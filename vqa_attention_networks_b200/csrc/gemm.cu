@@ -51,8 +51,8 @@ static EncodeTiledFn encode_fn() {
 }
 
 // bf16 matrix with `inner` contiguous elements per row, `outer` rows, row pitch ld (elements)
-static int make_tmap(CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer, uint64_t ld,
-                     uint32_t box_inner, uint32_t box_outer, uint64_t batch, uint64_t bstride) {
+int make_tmap(CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer, uint64_t ld, uint32_t box_inner,
+              uint32_t box_outer, uint64_t batch, uint64_t bstride, CUtensorMapSwizzle swizzle) {
   EncodeTiledFn fn = encode_fn();
   if (!fn) return set_error(VQA_B200_EDRIVER, "cuTensorMapEncodeTiled entry point not available");
   if (!aligned16(base) || (ld * 2) % 16 != 0)
@@ -68,7 +68,7 @@ static int make_tmap(CUtensorMap* map, const void* base, uint64_t inner, uint64_
   cuuint32_t box[3] = {box_inner, box_outer, 1};
   cuuint32_t estr[3] = {1, 1, 1};
   CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return set_error(VQA_B200_EDRIVER, "cuTensorMapEncodeTiled failed (%d)", (int)r);
   return 0;

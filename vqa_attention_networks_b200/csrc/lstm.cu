@@ -4,8 +4,9 @@
 //
 // The recurrence is latency-bound: 2*Bt*4H*H flops per step (0.2 GFLOP at Bt=26, H=1024) behind a
 // grid-wide dependency per step.  The stock path pays two kernel launches per step (a tf32 GEMM and
-// an elementwise cell); here ONE persistent kernel per direction runs the whole sequence (forward: cooperative
-// launch; backward: clusters of 4 CTAs whose co-residency is checked with cudaOccupancyMaxActiveClusters):
+// an elementwise cell); here ONE persistent kernel per direction runs the whole sequence (forward: cooperative launch of
+// clusters of 4 CTAs sharing each fetch of h_{t-1} by TMA multicast; backward: clusters of 4 CTAs splitting the
+// contraction; co-residency of the clusters is checked with cudaOccupancyMaxActiveClusters):
 //   * H/8 CTAs (128 at H=1024, one per SM), each owning 8 hidden units = 32 rows of W_hh (forward)
 //     or, in the backward, a share of the contraction for the 8*CL units of its cluster (see
 //     lstm_bwd_cluster_kernel; the single-CTA lstm_bwd_kernel is the fallback when clusters do not fit);
@@ -31,6 +32,7 @@
 #include <cuda_bf16.h>
 
 #include <stdlib.h>
+#include <string.h>
 
 #include "common.h"
 #include "ptx.cuh"
@@ -108,8 +110,10 @@ __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefe
 __device__ __forceinline__ float sigmoidf_(float x) { return __fdividef(1.f, 1.f + __expf(-x)); }
 __device__ __forceinline__ float tanhf_(float x) { return 1.f - __fdividef(2.f, 1.f + __expf(2.f * x)); }
 
-// Debug hooks (tools/gpu_lstm_phase_probe.py): per-phase cycle counters of CTA 0 / thread 0 and experiment switches.
+// Debug hooks (tools/lstm_phase_probe.py): per-phase cycle counters of thread 0 of the first g_dbg_ctas CTAs (16 per
+// CTA: [0..7] forward, [8..15] backward) and experiment switches.
 unsigned long long* g_dbg = nullptr;
+int g_dbg_ctas = 1;
 int g_mode = 0;
 int g_bwd_cluster = 0;      // 0 = auto (4, then 2, then 1), else forced cluster size (debug / A-B timing)
 enum { MODE_NOMMA = 2 };   // experiment switch: skip the MMAs (results are wrong; timing only)
@@ -153,7 +157,7 @@ __device__ __forceinline__ float ld_dsmem_f32(const float* local_ptr, uint32_t r
 }
 
 #ifdef VQA_B200_DEBUG
-#define LSTM_PROF(a) ((a).dbg != nullptr && blockIdx.x == 0 && tid == 0)
+#define LSTM_PROF(a) ((a).dbg != nullptr && (int)blockIdx.x < (a).dbg_ctas && tid == 0)
 #else
 #define LSTM_PROF(a) false      /* release kernels carry no phase counters: every `if (prof)` is dead code */
 #endif
@@ -250,6 +254,60 @@ __device__ __forceinline__ int sweep_mma(float (&acc)[2][NT][4], const uint32_t 
   }
 }
 
+// Byte offset of 16-byte chunk c of row r in a TMA box of RB-byte rows written with SWIZZLE_<RB>B (box base 1024-byte
+// aligned): bits [4, 4 + log2(RB/16)) of the offset are XORed with the bits above bit 7.
+template <int RB>
+__device__ __forceinline__ uint32_t swz(int r, int c) {
+  const uint32_t o = (uint32_t)(r * RB + c * 16);
+  return o ^ (((o >> 7) & (uint32_t)(RB / 16 - 1)) << 4);
+}
+
+// The multicast counterpart of sweep_mma: the warp's slice arrives by TMA in NH boxes (column halves, RB bytes per row,
+// 32-row tiles) that complete `full[hf]`; the MMAs run in exactly sweep_mma's order on exactly its operands, so the
+// accumulators are bit-identical.  Returns whether any operand still held the 0xFFFF sentinel.
+template <int KSTEPS, int NT>
+__device__ __forceinline__ bool mcast_mma(float (&acc)[2][NT][4], const uint32_t (&wfr)[KSTEPS][NT][2],
+                                          const unsigned char* stage, uint64_t* full, uint32_t phase, int Bt, int lane,
+                                          bool skip_mma) {
+  constexpr int NH = KSTEPS >= 2 ? 2 : 1;
+  constexpr int KH = KSTEPS / NH;
+  constexpr int RB = KH * 32;
+  const int lm_row = (lane & 7) + (((lane >> 3) & 1) << 3);
+  const int lm_c = lane >> 4;
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) acc[mt][nt][e] = 0.f;
+  uint32_t top = 0u;
+#pragma unroll
+  for (int hf = 0; hf < NH; ++hf) {
+    mbar_wait(full + hf, phase);
+    const unsigned char* tile = stage + hf * 32 * RB;
+    uint32_t afr[KH][2][4];
+#pragma unroll
+    for (int ks = 0; ks < KH; ++ks)
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+        if (mt * 16 < Bt) {
+          ldmatrix_x4(afr[ks][mt], tile + swz<RB>(mt * 16 + lm_row, ks * 2 + lm_c));
+          top = __vimax3_u16x2(top, afr[ks][mt][0], afr[ks][mt][1]);
+          top = __vimax3_u16x2(top, afr[ks][mt][2], afr[ks][mt][3]);
+        }
+    if (!skip_mma)
+#pragma unroll
+    for (int ks = 0; ks < KH; ++ks)
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+        if (mt * 16 < Bt)
+#pragma unroll
+          for (int nt = 0; nt < NT; ++nt)
+            mma16816(acc[mt][nt], afr[ks][mt], wfr[hf * KH + ks][nt][0], wfr[hf * KH + ks][nt][1]);
+  }
+  return __any_sync(0xFFFFFFFFu, sentinel_lanes(top) != 0u);
+}
+
 struct LstmFwdArgs {
   float* gates;                // in: x W_ih^T + b_ih + b_hh  [S, Bt, 4H]; out (training): activated gates i,f,g,o
   const __nv_bfloat16* whh;    // [4H, H]
@@ -257,29 +315,76 @@ struct LstmFwdArgs {
   __nv_bfloat16* hb;           // exchange buffer [S+1, Bt, H]: hb[0] = h_{-1} = 0, hb[1..] = 0xFFFF sentinels on entry
   float* c_all;                // [S, Bt, H] cell states (training) or nullptr
   int S, Bt, H;
-  unsigned long long* dbg;     // optional phase counters (debug): [0..7] forward, [8..15] backward
+  unsigned long long* dbg;     // optional phase counters (debug): 16 per CTA, [0..7] forward, [8..15] backward
+  int dbg_ctas;                // CTAs whose thread 0 records them (the rows dbg holds)
   int mode;
   LstmDrop drop;               // dropout applied to `out` only
+};
+
+// Shared memory of the forward kernel.  CL == 1 (sweep): one padded tile per warp, then the partial tiles.  CL > 1
+// (multicast): 1024-byte aligned TMA tiles [step parity][warp][column half] of 32 rows x RB bytes, the partial tiles,
+// the `full` barriers [parity][warp][half] and the `empty` barriers [warp].
+template <int KS, int CL>
+struct FwdSmem {
+  static constexpr int NH = KS >= 2 ? 2 : 1;
+  static constexpr int RB = KS / NH * 32;                  // bytes per row of one TMA box
+  static constexpr int TILE = 32 * RB;                     // bytes of one box tile
+  static constexpr size_t STAGE = CL == 1 ? (size_t)kWarps * kRows * (KS * 16 + 8) * 2 : (size_t)2 * kWarps * NH * TILE;
+  static constexpr size_t RED = STAGE;
+  static constexpr size_t BARS = RED + (size_t)kWarps * 32 * 40 * 4;
+  static constexpr size_t BYTES = CL == 1 ? BARS : BARS + (size_t)(2 * kWarps * NH + kWarps) * 8 + 1024;
 };
 
 // KS = k-steps (of 16) of one warp's contraction slice: H = 128 * KS.
 // Tile orientation: M = batch rows (2 m-tiles), N = the CTA's 32 gate rows in the order n = 4*unit + gate, so that the
 // four gate pre-activations of one (row, unit) are adjacent in the partial tiles (one 128-bit read per warp-partial).
-template <int KS>
-__global__ void __launch_bounds__(kThreads, 1) lstm_fwd_kernel(const LstmFwdArgs a) {
+//
+// CL > 1: multicast exchange.  The grid runs in clusters of CL CTAs, and warp w's slice of h_{t-1} (the same bytes for
+// every CTA) is fetched ONCE per cluster: warp w of the cluster's rank w % CL CTA (the slice's owner) polls the slice's
+// producers exactly as the sweep does, then issues the slice's TMA boxes multicast to the whole cluster; warp w of every
+// CTA waits on its own `full` barrier.  L2 reads and polls per step drop by the factor CL.  Every CTA receives the same
+// bytes, so all of them reach the same verdict on the sentinel check: on a hit each CTA re-arms its barrier and tells the
+// owner (remote arrive on the owner's `empty` barrier) that it is done reading the buffer, and the owner re-issues the
+// load once all CL have done so.
+// Buffers alternate by step parity.  The multicast of step t + 2 into a peer's parity-(t & 1) tile cannot overtake that
+// peer's reads of step t: the owner issues it only after it has seen h_{t+1} of the slice's producers, those needed the
+// peer's h_t, and the peer publishes h_t after the __syncthreads that follows every one of its warps' reads of step t.
+template <int KS, int CL>
+__global__ void __launch_bounds__(kThreads, 1) lstm_fwd_kernel(const LstmFwdArgs a, const __grid_constant__ CUtensorMap hmap) {
+  using SM = FwdSmem<KS, CL>;
   constexpr int PITCH = KS * 16 + 8;     // bf16 elements; (PITCH/2) % 8 == 4 -> conflict-free ldmatrix
   constexpr int RP = 40;                 // floats per batch row of a partial tile: 8*b + n is conflict-free
   constexpr int NPROD = 2 * KS;          // CTAs that produce one warp's slice of h
+  constexpr int NH = SM::NH;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  __nv_bfloat16* hs = reinterpret_cast<__nv_bfloat16*>(smem_raw);
-  float* red = reinterpret_cast<float*>(smem_raw + (size_t)kWarps * kRows * PITCH * 2);
+  unsigned char* smem = CL == 1 ? smem_raw : smem_raw + ((1024u - (s_u32(smem_raw) & 1023u)) & 1023u);
+  __nv_bfloat16* hs = reinterpret_cast<__nv_bfloat16*>(smem);
+  float* red = reinterpret_cast<float*>(smem + SM::RED);
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + SM::BARS);
+  uint64_t* empty = full + 2 * kWarps * NH;
 
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, g = lane >> 2, tg = lane & 3;
   const int H = a.H, Bt = a.Bt;
   const int j0 = blockIdx.x * kU;
   const int kw = w * KS * 16;            // first contraction index of this warp
+  const uint32_t owner = (uint32_t)(w % CL);
+  const bool own = CL > 1 && cluster_rank() == owner;
 
-  for (int i = tid; i < kWarps * kRows * PITCH / 2; i += kThreads) reinterpret_cast<uint32_t*>(hs)[i] = 0u;
+  // rows >= Bt of the tiles are never written and must read as zero
+  for (int i = tid; i < (int)(SM::STAGE / 4); i += kThreads) reinterpret_cast<uint32_t*>(hs)[i] = 0u;
+  if constexpr (CL > 1) {
+    if (tid == 0) {
+      for (int i = 0; i < 2 * kWarps * NH; ++i) mbar_init(full + i, 1);
+      for (int i = 0; i < kWarps; ++i) mbar_init(empty + i, CL);
+      fence_mbar_init();
+    }
+    fence_proxy_async_smem();
+    __syncthreads();
+    if (lane == 0)
+      for (int i = 0; i < 2 * NH; ++i) mbar_expect_tx(full + ((i / NH) * kWarps + w) * NH + i % NH, (uint32_t)(Bt * SM::RB));
+    if (own && lane == 0) tma_prefetch_desc(&hmap);
+    cluster_barrier();                   // every barrier of the cluster is armed before the first multicast lands
+  }
 
   // W_hh slice as B fragments: column n = nt*8 + g of the tile is gate (n & 3) of unit (n >> 2)
   uint32_t wfr[KS][4][2];
@@ -311,17 +416,48 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_fwd_kernel(const LstmFwdArgs
     for (int q = 0; q < 4; ++q) xq[q] = __ldcs(gp0 + (size_t)q * H);
   }
 
+  uint32_t ph = 0u, eph = 0u;           // multicast: phase bits of the warp's `full` barriers (bit = parity), `empty`
   for (int t = 0; t < a.S; ++t) {
     if (prof) tk = clock64();
     const __nv_bfloat16* src = a.hb + (size_t)t * Bt * H + kw;
     // ---- wait for h_{t-1}: each lane watches the LAST row's piece of one producer CTA of this warp's slice
-    if (t > 0) {
+    if (t > 0 && (CL == 1 || own)) {
       if (lane < NPROD) spin_piece(src + (size_t)(Bt - 1) * H + lane * 8);
       __syncwarp();
     }
     LSTM_TICK(0)
     float acc[2][4][4];
-    const int tries = sweep_mma<KS, 4>(acc, wfr, hw, src, (size_t)H, Bt, lane, (a.mode & MODE_NOMMA) != 0);
+    int tries = 0;
+    if constexpr (CL == 1) {
+      tries = sweep_mma<KS, 4>(acc, wfr, hw, src, (size_t)H, Bt, lane, (a.mode & MODE_NOMMA) != 0);
+    } else {
+      const int p = t & 1;
+      unsigned char* tiles = smem + (size_t)(p * kWarps + w) * NH * SM::TILE;
+      uint64_t* fb = full + (p * kWarps + w) * NH;
+      auto issue = [&]() {
+        if (own && lane == 0)
+#pragma unroll
+          for (int hf = 0; hf < NH; ++hf)
+            tma_load_3d_multicast(tiles + hf * SM::TILE, &hmap, fb + hf, kw + hf * (KS / NH) * 16, t * Bt, 0,
+                                  (uint16_t)((1u << CL) - 1u));
+      };
+      issue();
+      for (;;) {
+        const bool bad = mcast_mma<KS, 4>(acc, wfr, tiles, fb, (ph >> p) & 1u, Bt, lane, (a.mode & MODE_NOMMA) != 0);
+        ph ^= 1u << p;
+        if (lane == 0)                   // arm the next delivery into this buffer: the retry, or step t + 2
+          for (int hf = 0; hf < NH; ++hf) mbar_expect_tx(fb + hf, (uint32_t)(Bt * SM::RB));
+        if (!bad) break;
+        if (++tries > (1 << 22)) __trap();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_cluster(empty + w, owner);
+        if (own) {
+          mbar_wait(empty + w, eph);
+          eph ^= 1u;
+          issue();
+        }
+      }
+    }
     if (prof) pc[7] += tries;
     LSTM_TICK(1)
 #pragma unroll
@@ -371,8 +507,9 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_fwd_kernel(const LstmFwdArgs
     __syncthreads();               // the partial tiles are re-written by the next step's MMAs
     LSTM_TICK(6)
   }
+  if constexpr (CL > 1) cluster_barrier();   // no CTA exits while its multicasts or a peer's arrives may be in flight
   if (prof)
-    for (int i = 0; i < 8; ++i) a.dbg[i] = (unsigned long long)pc[i];
+    for (int i = 0; i < 8; ++i) a.dbg[(size_t)blockIdx.x * 16 + i] = (unsigned long long)pc[i];
 }
 
 struct LstmBwdArgs {
@@ -383,6 +520,7 @@ struct LstmBwdArgs {
   __nv_bfloat16* dg;             // exchange buffer + result: dL/d(pre-activation gates) [S, Bt, 4H], 0xFFFF on entry
   int S, Bt, H;
   unsigned long long* dbg;
+  int dbg_ctas;
   int mode;
   long long dout_st, dout_sb;    // strides of dout in elements (the gradient arrives in the caller's [Bt, S, H] order)
   int w_layout;
@@ -550,7 +688,7 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_bwd_kernel(const LstmBwdArgs
     LSTM_TICK(6)
   }
   if (prof)
-    for (int i = 0; i < 8; ++i) a.dbg[8 + i] = (unsigned long long)pc[i];
+    for (int i = 0; i < 8; ++i) a.dbg[(size_t)blockIdx.x * 16 + 8 + i] = (unsigned long long)pc[i];
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -701,21 +839,89 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_bwd_cluster_kernel(const Lst
   __syncthreads();
   cluster_barrier();                     // nobody exits while a peer may still read its shared memory
   if (prof)
-    for (int i = 0; i < 8; ++i) a.dbg[8 + i] = (unsigned long long)pc[i];
+    for (int i = 0; i < 8; ++i) a.dbg[(size_t)blockIdx.x * 16 + 8 + i] = (unsigned long long)pc[i];
 }
 
 #undef LSTM_TICK
 
-template <int KS>
+// Whether cluster launches of the recurrence are also cooperative.  ncu's kernel replay refuses cooperative cluster
+// launches (LaunchFailed): VQA_B200_LSTM_COOP=0 drops the attribute for profiling runs on an otherwise idle GPU.
+bool coop_launch() {
+  static int coop = -1;
+  if (coop < 0) {
+    const char* e = getenv("VQA_B200_LSTM_COOP");
+    coop = (e && e[0] == '0') ? 0 : 1;
+  }
+  return coop != 0;
+}
+
+// CL == 1: the sweep form, a cooperative launch.  CL > 1: the multicast form, a cooperative cluster launch; returns
+// -1000 when CL-CTA clusters cannot all be co-resident on this device (caller falls back).
+template <int KS, int CL>
 int launch_fwd(const LstmFwdArgs& a, cudaStream_t st) {
-  constexpr int PITCH = KS * 16 + 8;
-  const size_t smem = (size_t)kWarps * kRows * PITCH * 2 + (size_t)kWarps * 32 * 40 * 4;
-  VQA_CUDA_CHECK(cudaFuncSetAttribute(lstm_fwd_kernel<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  using SM = FwdSmem<KS, CL>;
+  auto kern = lstm_fwd_kernel<KS, CL>;
+  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::BYTES));
   LstmFwdArgs args = a;
-  void* params[] = {&args};
-  VQA_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)lstm_fwd_kernel<KS>, dim3(a.H / kU), dim3(kThreads), params,
-                                             smem, st));
+  CUtensorMap hmap;
+  memset(&hmap, 0, sizeof(hmap));
+  if (CL == 1) {
+    void* params[] = {&args, &hmap};
+    VQA_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)kern, dim3(a.H / kU), dim3(kThreads), params, SM::BYTES, st));
+    return 0;
+  }
+  // hb as a [(S+1) * Bt, H] matrix (a batch of one); one box = one column half of a warp's slice over the Bt rows of a step
+  constexpr CUtensorMapSwizzle swz_mode = SM::RB == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                          : SM::RB == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
+  if (int rc = make_tmap(&hmap, a.hb, (uint64_t)a.H, (uint64_t)(a.S + 1) * a.Bt, (uint64_t)a.H, (uint32_t)(SM::RB / 2),
+                         (uint32_t)a.Bt, 1, 0, swz_mode))
+    return rc;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(a.H / kU);
+  cfg.blockDim = dim3(kThreads);
+  cfg.dynamicSmemBytes = SM::BYTES;
+  cfg.stream = st;
+  cudaLaunchAttribute attrs[2];
+  attrs[0].id = cudaLaunchAttributeClusterDimension;
+  attrs[0].val.clusterDim.x = CL;
+  attrs[0].val.clusterDim.y = 1;
+  attrs[0].val.clusterDim.z = 1;
+  cfg.attrs = attrs;
+  cfg.numAttrs = 1;
+  int nclusters = 0;
+  if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess) {
+    (void)cudaGetLastError();
+    return -1000;
+  }
+  if (nclusters * CL < a.H / kU) return -1000;
+  attrs[1].id = cudaLaunchAttributeCooperative;   // see launch_bwd_cluster
+  attrs[1].val.cooperative = 1;
+  cfg.numAttrs = coop_launch() ? 2 : 1;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args, hmap);
+  if (e != cudaSuccess) return set_error((int)e, "lstm_fwd cluster launch: %s", cudaGetErrorString(e));
   return 0;
+}
+
+// Exchange of the forward: VQA_B200_LSTM_EXCHANGE = sweep | multicast (read per call: tests compare the two), multicast
+// by default; VQA_B200_LSTM_FWD_CLUSTER = 2 | 4 forces the cluster size of the multicast form, otherwise (or 0)
+// clusters of 4, then 2, whichever can be co-resident, and the sweep form when neither can.
+template <int KS>
+int launch_fwd_any(const LstmFwdArgs& a, cudaStream_t st) {
+  bool mcast = true;
+  if (const char* e = getenv("VQA_B200_LSTM_EXCHANGE")) {
+    if (strcmp(e, "sweep") == 0) mcast = false;
+    else if (strcmp(e, "multicast") != 0)
+      return set_error(VQA_B200_EINVAL, "VQA_B200_LSTM_EXCHANGE must be sweep or multicast (got '%s')", e);
+  }
+  int forced = 0;
+  if (const char* e = getenv("VQA_B200_LSTM_FWD_CLUSTER")) forced = atoi(e);
+  int rc = -1000;
+  if (mcast) {
+    if (forced == 4 || forced == 0) rc = launch_fwd<KS, 4>(a, st);
+    if (rc == -1000 && (forced == 2 || forced == 0)) rc = launch_fwd<KS, 2>(a, st);
+  }
+  if (rc == -1000) rc = launch_fwd<KS, 1>(a, st);
+  return rc;
 }
 
 template <int KS>
@@ -760,14 +966,8 @@ int launch_bwd_cluster(const LstmBwdArgs& a, cudaStream_t st) {
   // Co-residency of the whole grid is required (CTAs wait on each other).  The occupancy query above answers for an
   // idle GPU only; under data-parallel training the gradient all-reduce may already hold SMs when this kernel is
   // enqueued, so the launch is COOPERATIVE as well: the grid is only started once all of it fits, instead of resident
-  // CTAs spinning on peers that cannot be scheduled.  ncu's kernel replay refuses cooperative cluster launches
-  // (LaunchFailed): VQA_B200_LSTM_COOP=0 drops the attribute for profiling runs on an otherwise idle GPU.
-  static int coop = -1;
-  if (coop < 0) {
-    const char* e = getenv("VQA_B200_LSTM_COOP");
-    coop = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (coop) {
+  // CTAs spinning on peers that cannot be scheduled.
+  if (coop_launch()) {
     attrs[1].id = cudaLaunchAttributeCooperative;
     attrs[1].val.cooperative = 1;
     cfg.numAttrs = 2;
@@ -811,6 +1011,8 @@ extern "C" void vqa_b200_debug_set_lstm(void* device_u64x16, int mode) {
   g_dbg = (unsigned long long*)device_u64x16;
   g_mode = mode & 0xFF;
   g_bwd_cluster = (mode >> 8) & 0xF;   // bits 8..11: force the backward cluster size (1, 2, 4); 0 = auto
+  g_dbg_ctas = (mode >> 16) & 0xFFFF;  // bits 16..31: CTAs (rows of 16 counters) the buffer holds; 0 = CTA 0 only
+  if (g_dbg_ctas < 1) g_dbg_ctas = 1;
 }
 #endif
 
@@ -941,14 +1143,14 @@ extern "C" int vqa_b200_lstm_fwd(float* gates, const void* whh, float* out, void
   if (int rc = check_shape("lstm_fwd", S, Bt, H)) return rc;
   if (!gates || !whh || !out || !hb) return set_error(VQA_B200_EINVAL, "lstm_fwd: null pointer");
   if (!aligned16(whh) || !aligned16(hb)) return set_error(VQA_B200_EALIGN, "lstm_fwd: whh / hb must be 16-byte aligned");
-  LstmFwdArgs a{gates, (const __nv_bfloat16*)whh, out, (__nv_bfloat16*)hb, c_all, S, Bt, H, g_dbg, g_mode,
+  LstmFwdArgs a{gates, (const __nv_bfloat16*)whh, out, (__nv_bfloat16*)hb, c_all, S, Bt, H, g_dbg, g_dbg_ctas, g_mode,
                 make_drop(drop_p, seed, seed_dev)};
   cudaStream_t st = (cudaStream_t)stream;
   switch (H / 128) {
-    case 1: return launch_fwd<1>(a, st);
-    case 2: return launch_fwd<2>(a, st);
-    case 4: return launch_fwd<4>(a, st);
-    default: return launch_fwd<8>(a, st);
+    case 1: return launch_fwd_any<1>(a, st);
+    case 2: return launch_fwd_any<2>(a, st);
+    case 4: return launch_fwd_any<4>(a, st);
+    default: return launch_fwd_any<8>(a, st);
   }
 }
 
@@ -961,7 +1163,7 @@ extern "C" int vqa_b200_lstm_bwd(const float* gates, const float* c_all, const f
   if (!aligned16(whh) || !aligned16(dg)) return set_error(VQA_B200_EALIGN, "lstm_bwd: whh / dg must be 16-byte aligned");
   if (w_layout != 0 && w_layout != 1) return set_error(VQA_B200_EINVAL, "lstm_bwd: w_layout must be 0 ([H,4H]) or 1 ([4H,H])");
   if (dout_st <= 0 && S > 1) return set_error(VQA_B200_EINVAL, "lstm_bwd: bad dout strides");
-  LstmBwdArgs a{gates, c_all, dout, (const __nv_bfloat16*)whh, (__nv_bfloat16*)dg, S, Bt, H, g_dbg, g_mode,
+  LstmBwdArgs a{gates, c_all, dout, (const __nv_bfloat16*)whh, (__nv_bfloat16*)dg, S, Bt, H, g_dbg, g_dbg_ctas, g_mode,
                 (long long)dout_st, (long long)dout_sb, w_layout, make_drop(drop_p, seed, seed_dev)};
   cudaStream_t st = (cudaStream_t)stream;
   switch (H / 128) {

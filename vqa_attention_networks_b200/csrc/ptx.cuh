@@ -79,6 +79,17 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
+// 3-D tiled load multicast to the CTAs of the cluster in `cta_mask`: ONE read of the box lands at the same shared-memory
+// offset in every one of them and completes the transaction bytes on the barrier at the same offset in each.
+__device__ __forceinline__ void tma_load_3d_multicast(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0,
+                                                      int c1, int c2, uint16_t cta_mask) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, "
+      "%4, %5}], [%2], %6;" ::"r"(smem_u32(smem_dst)),
+      "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask)
+      : "memory");
+}
+
 // 3-D tiled load (c2 = batch index); every operand of the GEMM kernel is described as [batch, outer, inner].
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
                                             int c2) {
