@@ -1,5 +1,7 @@
 """Per-phase cycle counters of the recurrence kernels over ALL CTAs, on config 2's shape (S=256 steps over Bt=26 rows,
-300 -> 1024), forward (training form) and backward, for each forward exchange form (sweep / multicast).
+300 -> 1024), forward (training form) and backward, for each backward launch form: unsplit clusters of 4 (`rows1`)
+and the row split (`rows2`), forced through the debug hook's mode bits 12..13.  The forward runs in its default form
+(VQA_B200_LSTM_EXCHANGE selects another one).
 
 Builds the library with VQA_B200_DEBUG=1 (instrumented kernels + the vqa_b200_debug_set_lstm hook) into a temporary
 copy of the package, so the tree's release library is left alone.  Thread 0 of every CTA accumulates clock64() deltas
@@ -81,9 +83,9 @@ def main():
         dbg = torch.zeros(ncta * 16, dtype=torch.int64, device=dev)
         res = {"card": card(), "shape": {"S": S, "Bt": Bt, "E": E, "H": H}, "unit": "SM cycles (clock64)",
                "note": "thread 0 of every CTA; forward and backward of the last of 5 fwd+bwd calls"}
-        for mode in ("sweep", "multicast"):
-            os.environ["VQA_B200_LSTM_EXCHANGE"] = mode
-            L.vqa_b200_debug_set_lstm(ctypes_ptr(dbg), ncta << 16)
+        for rows in (1, 2):
+            mode = "rows%d" % rows
+            L.vqa_b200_debug_set_lstm(ctypes_ptr(dbg), (ncta << 16) | (rows << 12))
             for _ in range(5):
                 for t in (x, W_ih, W_hh, b):
                     t.grad = None
@@ -94,7 +96,6 @@ def main():
             res[mode] = {"forward": summarise(rows[:, :8], FWD_PHASES, S),
                          "backward": summarise(rows[:, 8:], BWD_PHASES, S - 1)}
             print(mode, json.dumps(res[mode]), flush=True)
-        os.environ.pop("VQA_B200_LSTM_EXCHANGE", None)
         print(json.dumps(res, indent=1))
         if dst:
             d = os.path.dirname(dst)

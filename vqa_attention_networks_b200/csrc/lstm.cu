@@ -6,10 +6,12 @@
 // grid-wide dependency per step.  The stock path pays two kernel launches per step (a tf32 GEMM and
 // an elementwise cell); here ONE persistent kernel per direction runs the whole sequence (forward: cooperative launch of
 // clusters of 4 CTAs sharing each fetch of h_{t-1} by TMA multicast; backward: clusters of 4 CTAs splitting the
-// contraction; co-residency of the clusters is checked with cudaOccupancyMaxActiveClusters):
+// contraction, each half of the grid running half of the batch rows; co-residency of the clusters is checked with
+// cudaOccupancyMaxActiveClusters):
 //   * H/8 CTAs (128 at H=1024, one per SM), each owning 8 hidden units = 32 rows of W_hh (forward)
-//     or, in the backward, a share of the contraction for the 8*CL units of its cluster (see
-//     lstm_bwd_cluster_kernel; the single-CTA lstm_bwd_kernel is the fallback when clusters do not fit);
+//     or, in the backward, a share of the contraction for the 64 units of its cluster over half of the rows (see
+//     lstm_bwd_rows_kernel; lstm_bwd_cluster_kernel, 8*CL units over all rows, and the single-CTA lstm_bwd_kernel
+//     are the fallbacks when it does not fit or Bt = 1);
 //   * the CTA's slice of W_hh lives in REGISTERS for the whole sequence, already laid out as
 //     mma.sync.m16n8k16 operand fragments (8 warps split the contraction; 64 registers per thread);
 //   * the step-to-step exchange (h_t forward, dgates_t backward; bf16, through L2) carries its own
@@ -116,6 +118,7 @@ unsigned long long* g_dbg = nullptr;
 int g_dbg_ctas = 1;
 int g_mode = 0;
 int g_bwd_cluster = 0;      // 0 = auto (4, then 2, then 1), else forced cluster size (debug / A-B timing)
+int g_bwd_rows = 0;         // 0 = auto, 1 = unsplit backward forms, 2 = row-split form (debug / A-B timing)
 enum { MODE_NOMMA = 2 };   // experiment switch: skip the MMAs (results are wrong; timing only)
 
 __device__ __forceinline__ uint32_t cluster_rank() {
@@ -190,13 +193,14 @@ LstmDrop make_drop(float p, uint32_t seed, const uint32_t* seed_dev) {
 //   X      : rows of the exchange buffer (bf16, `src` = first column of the slice, `src_pitch` elements between rows);
 //            pulled out of L2 with cp.async.cg in (up to) two column halves so that the tensor cores start on the
 //            first half while the second is still in flight; staged in the warp's private shared-memory tile
-//   Wslice : resident in registers as mma.m16n8k16 B fragments (wfr)
-// The A fragments ldmatrix returns are checked for the 0xFFFF "not written yet" mark; returns the number of repeated
-// sweeps (0 in the common case).
-template <int KSTEPS, int NT>
-__device__ __forceinline__ int sweep_mma(float (&acc)[2][NT][4], const uint32_t (&wfr)[KSTEPS][NT][2],
+//   Wslice : mma.m16n8k16 B fragments, n-tiles [0, NTR) resident in registers (wfr), n-tiles [NTR, NT) in shared
+//            memory (wsm, [ks][nt - NTR][lane] as uint2: one conflict-free 8-byte load per lane)
+// MT m-tiles of 16 rows (Bt <= 16 * MT).  The A fragments ldmatrix returns are checked for the 0xFFFF "not written yet"
+// mark; returns the number of repeated sweeps (0 in the common case).
+template <int KSTEPS, int NT, int MT, int NTR>
+__device__ __forceinline__ int sweep_mma(float (&acc)[MT][NT][4], const uint32_t (&wfr)[KSTEPS][NTR][2],
                                          __nv_bfloat16* stage, const __nv_bfloat16* src, size_t src_pitch, int Bt,
-                                         int lane, bool skip_mma) {
+                                         int lane, bool skip_mma, const uint2* wsm = nullptr) {
   constexpr int PITCH = KSTEPS * 16 + 8;
   constexpr int NH = KSTEPS >= 2 ? 2 : 1;
   constexpr int KH = KSTEPS / NH;
@@ -214,12 +218,12 @@ __device__ __forceinline__ int sweep_mma(float (&acc)[2][NT][4], const uint32_t 
     for (int hf = 0; hf < NH; ++hf) {
 #pragma unroll
       for (int j = 0; j < PR; ++j)
-        if (prow + j * RPI < Bt)
+        if (j * RPI < MT * 16 && prow + j * RPI < Bt)
           cp_async16(sdst + j * RPI * PITCH + hf * KH * 16, gsrc + (size_t)(j * RPI) * src_pitch + hf * KH * 16);
       cp_async_commit();
     }
 #pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
+    for (int mt = 0; mt < MT; ++mt)
 #pragma unroll
       for (int nt = 0; nt < NT; ++nt)
 #pragma unroll
@@ -229,11 +233,11 @@ __device__ __forceinline__ int sweep_mma(float (&acc)[2][NT][4], const uint32_t 
     for (int hf = 0; hf < NH; ++hf) {
       if (hf == 0 && NH == 2) cp_async_wait<1>(); else cp_async_wait<0>();
       __syncwarp();
-      uint32_t afr[KH][2][4];
+      uint32_t afr[KH][MT][4];
 #pragma unroll
       for (int ks = 0; ks < KH; ++ks)
 #pragma unroll
-        for (int mt = 0; mt < 2; ++mt)
+        for (int mt = 0; mt < MT; ++mt)
           if (mt * 16 < Bt) {
             ldmatrix_x4(afr[ks][mt], stage + (mt * 16 + lm_row) * PITCH + (hf * KH + ks) * 16 + lm_k);
             top = __vimax3_u16x2(top, afr[ks][mt][0], afr[ks][mt][1]);
@@ -243,11 +247,18 @@ __device__ __forceinline__ int sweep_mma(float (&acc)[2][NT][4], const uint32_t 
 #pragma unroll
       for (int ks = 0; ks < KH; ++ks)
 #pragma unroll
-        for (int mt = 0; mt < 2; ++mt)
+        for (int mt = 0; mt < MT; ++mt)
           if (mt * 16 < Bt)
 #pragma unroll
-            for (int nt = 0; nt < NT; ++nt)
-              mma16816(acc[mt][nt], afr[ks][mt], wfr[hf * KH + ks][nt][0], wfr[hf * KH + ks][nt][1]);
+            for (int nt = 0; nt < NT; ++nt) {
+              if (nt < NTR) {
+                mma16816(acc[mt][nt], afr[ks][mt], wfr[hf * KH + ks][nt < NTR ? nt : 0][0],
+                         wfr[hf * KH + ks][nt < NTR ? nt : 0][1]);
+              } else {
+                const uint2 b = wsm[((hf * KH + ks) * (NT - NTR) + (nt - NTR)) * 32 + lane];
+                mma16816(acc[mt][nt], afr[ks][mt], b.x, b.y);
+              }
+            }
     }
     if (!__any_sync(0xFFFFFFFFu, sentinel_lanes(top) != 0u)) return tries;
     if (++tries > (1 << 22)) __trap();
@@ -842,6 +853,185 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_bwd_cluster_kernel(const Lst
     for (int i = 0; i < 8; ++i) a.dbg[(size_t)blockIdx.x * 16 + 8 + i] = (unsigned long long)pc[i];
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Backward recurrence, row-split version.  A cluster reads Bt * 4H * 2 bytes of dgates_t per step whatever it does
+// inside, since it contracts over all 4H gate columns for the units it owns; total L2 traffic per step is that times
+// the number of clusters, i.e. inversely proportional to the units a cluster owns.  The Bt batch rows are independent
+// recurrences, so the grid is split into two halves that each run half of the rows: cluster (G, h) of 4 CTAs owns the
+// 64 units [64G, 64G + 64) for row half h (rows [0, ceil(Bt/2)) or [ceil(Bt/2), Bt)), which halves the L2 reads and the
+// producers a warp polls against lstm_bwd_cluster_kernel<KS, 4>.  CTA rank r contracts over gate plane r exactly as
+// there (same k-slice per warp, same MMA k order, same warp- and rank-sum order, dh starting from the same masked dout),
+// computes partial sums for the 64 units over one 16-row m-tile, and owns 16 units for the gate math and publication
+// (two 16-byte pieces per gate plane and row).  A row's element is computed the same way whichever m-tile row or n-tile
+// column it sits in, so dgates are bit-identical to the unsplit form.
+// Each warp holds B fragments for 8 n-tiles; where they do not all fit in registers (KS = 8) n-tiles 4..7 live in
+// shared memory in lane order.
+// ---------------------------------------------------------------------------------------------------------------
+template <int KS>
+struct BwdRowsSmem {
+  static constexpr int NTR = KS <= 4 ? 8 : 4;       // n-tiles whose B fragments stay in registers
+  static constexpr int PITCH = KS * 16 + 8;         // bf16 elements per operand tile row (conflict-free ldmatrix)
+  static constexpr int RP = 64 + 8;                 // floats per row of the partial tiles (conflict-free, see below)
+  static constexpr size_t RED = (size_t)kWarps * 16 * PITCH * 2;          // after the operand tiles [warp][16][PITCH]
+  static constexpr size_t PART = RED + (size_t)kWarps * 16 * RP * 4;      // after the warp partials [warp][16][RP]
+  static constexpr size_t WSM = PART + (size_t)2 * 16 * RP * 4;           // after the CTA partials [parity][16][RP]
+  static constexpr size_t BYTES = WSM + (size_t)kWarps * KS * (8 - NTR) * 32 * 8;   // B fragments [warp][ks][nt][lane]
+};
+
+template <int KS>
+__global__ void __launch_bounds__(kThreads, 1) lstm_bwd_rows_kernel(const LstmBwdArgs a) {
+  using SM = BwdRowsSmem<KS>;
+  constexpr int NTR = SM::NTR, PITCH = SM::PITCH, RP = SM::RP;
+  constexpr int NPROD = 2 * KS;          // 16-byte pieces of one row of a warp's slice (two per producer CTA)
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __nv_bfloat16* ds = reinterpret_cast<__nv_bfloat16*>(smem_raw);
+  float* red = reinterpret_cast<float*>(smem_raw + SM::RED);
+  float* part = reinterpret_cast<float*>(smem_raw + SM::PART);
+
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, g = lane >> 2, tg = lane & 3;
+  const int H = a.H, Bt = a.Bt, S = a.S;
+  const uint32_t rank = cluster_rank();
+  const int ng = H / 64;                             // unit groups per row half
+  const int cid = blockIdx.x / 4;
+  const int u0 = (cid % ng) * 64;                    // first unit of the cluster
+  const int j0 = u0 + (int)rank * 16;                // own units (gate math, dgates output)
+  const int rh = (Bt + 1) / 2;
+  const int r0 = cid < ng ? 0 : rh, nr = cid < ng ? rh : Bt - rh;   // the cluster's rows
+  const int kw = (int)rank * H + w * KS * 16;        // first gate column of this warp's contraction slice
+
+  for (int i = tid; i < (int)(SM::RED / 4); i += kThreads) reinterpret_cast<uint32_t*>(ds)[i] = 0u;
+
+  // W_hh[k, u0 + nt*8 + g] for the warp's k-slice as B fragments (n = unit, k = gate column)
+  uint32_t bfr[KS][NTR][2];
+  uint2* wsm = reinterpret_cast<uint2*>(smem_raw + SM::WSM) + (size_t)w * KS * (8 - NTR) * 32;
+#pragma unroll
+  for (int ks = 0; ks < KS; ++ks) {
+    const size_t kq = (size_t)kw + ks * 16 + 2 * tg;
+#pragma unroll
+    for (int nt = 0; nt < NTR; ++nt) {
+      bfr[ks][nt][0] = ld_w_pair(a.whhT, a.w_layout, (size_t)(u0 + nt * 8 + g), kq, H);
+      bfr[ks][nt][1] = ld_w_pair(a.whhT, a.w_layout, (size_t)(u0 + nt * 8 + g), kq + 8, H);
+    }
+#pragma unroll
+    for (int nt = NTR; nt < 8; ++nt)
+      wsm[(ks * (8 - NTR) + nt - NTR) * 32 + lane] =
+          make_uint2(ld_w_pair(a.whhT, a.w_layout, (size_t)(u0 + nt * 8 + g), kq, H),
+                     ld_w_pair(a.whhT, a.w_layout, (size_t)(u0 + nt * 8 + g), kq + 8, H));
+  }
+  __syncthreads();
+
+  __nv_bfloat16* dw = ds + (size_t)w * 16 * PITCH;
+  float* redw = red + w * 16 * RP;
+  const int eb = tid >> 4, eu = tid & 15;            // gate-math role: (row of the half, unit)
+  const int b = r0 + eb;
+  const bool active = eb < nr;
+  // CTA-reduction role: row (tid >> 3) & 15, units (2 jj + (tid >> 7)) * 8 + (tid & 7): a warp reads 4 rows x 8 units,
+  // banks 8 * row + unit (RP % 32 == 8), conflict-free
+  const int qr = (tid >> 3) & 15, qu = ((tid >> 7) << 3) + (tid & 7);
+  float dc = 0.f;
+  const bool prof = LSTM_PROF(a);
+  long long pc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tk = 0;
+  const uint32_t dseed = a.drop.thresh16 ? effective_seed(a.drop.seed, a.drop.seed_dev) : 0u;
+
+  // saved activations pulled into L2 one step ahead (see lstm_bwd_cluster_kernel)
+  auto prefetch = [&](int t) {
+    const size_t row = (size_t)t * Bt + b;
+    const size_t o = row * H + j0 + eu;
+    const float* gp = a.gates + row * 4 * H + j0 + eu;
+    prefetch_l2(gp);
+    prefetch_l2(gp + (size_t)H);
+    prefetch_l2(gp + (size_t)2 * H);
+    prefetch_l2(gp + (size_t)3 * H);
+    prefetch_l2(a.c_all + o);
+    prefetch_l2(a.dout + (size_t)t * a.dout_st + (size_t)b * a.dout_sb + j0 + eu);
+  };
+  if (active && (eu & 7) == 0) prefetch(S - 1);
+  cluster_barrier();                     // every CTA of the cluster is resident before anyone touches remote smem
+
+  for (int t = S - 1; t >= 0; --t) {
+    if (prof) tk = clock64();
+    float gi = 0.f, gf = 0.f, gg = 0.f, go = 0.f, ct = 0.f, cprev = 0.f, dh = 0.f;
+    if (active) {
+      const size_t row = (size_t)t * Bt + b;
+      const size_t o = row * H + j0 + eu;
+      const float* gp = a.gates + row * 4 * H + j0 + eu;
+      gi = __ldcs(gp);
+      gf = __ldcs(gp + (size_t)H);
+      gg = __ldcs(gp + (size_t)2 * H);
+      go = __ldcs(gp + (size_t)3 * H);
+      ct = __ldcs(a.c_all + o);
+      cprev = t > 0 ? __ldcs(a.c_all + o - (size_t)Bt * H) : 0.f;
+      dh = drop_out(__ldcs(a.dout + (size_t)t * a.dout_st + (size_t)b * a.dout_sb + j0 + eu), a.drop, dseed,
+                    (uint32_t)row, (uint32_t)(j0 + eu));
+      if (t > 0 && (eu & 7) == 0) prefetch(t - 1);   // one lane per 32-byte sector
+    }
+    if (t < S - 1) {                     // uniform over the cluster
+      // the half's rows of dgates_{t+1}; canaries: the half's last row
+      const __nv_bfloat16* src = a.dg + ((size_t)(t + 1) * Bt + r0) * 4 * H + kw;
+#pragma unroll 1
+      for (int i = lane; i < NPROD; i += 32) spin_piece(src + (size_t)(nr - 1) * 4 * H + i * 8);
+      __syncwarp();
+      LSTM_TICK(0)
+      float acc[1][8][4];
+      const int tries =
+          sweep_mma<KS, 8>(acc, bfr, dw, src, (size_t)4 * H, nr, lane, (a.mode & MODE_NOMMA) != 0, wsm);
+      LSTM_TICK(1)
+      if (prof) pc[7] += tries;
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        const int uc = nt * 8 + 2 * tg;
+        *reinterpret_cast<float2*>(redw + g * RP + uc) = make_float2(acc[0][nt][0], acc[0][nt][1]);
+        *reinterpret_cast<float2*>(redw + (g + 8) * RP + uc) = make_float2(acc[0][nt][2], acc[0][nt][3]);
+      }
+      LSTM_TICK(2)
+      __syncthreads();
+      // this CTA's partial sums for all 64 units of the cluster, double-buffered by step parity (as in
+      // lstm_bwd_cluster_kernel)
+      float* pbuf = part + (t & 1) * 16 * RP;
+#pragma unroll
+      for (int jj = 0; jj < 4; ++jj) {
+        float sum = 0.f;
+#pragma unroll
+        for (int ww = 0; ww < kWarps; ++ww) sum += red[(ww * 16 + qr) * RP + jj * 16 + qu];
+        pbuf[qr * RP + jj * 16 + qu] = sum;
+      }
+      LSTM_TICK(3)
+      step_barrier();
+      if (active) {
+#pragma unroll
+        for (int rr = 0; rr < 4; ++rr) dh += ld_dsmem_f32(pbuf + eb * RP + (int)rank * 16 + eu, (uint32_t)rr);
+      }
+    }
+    float d_i = 0.f, d_f = 0.f, d_g = 0.f, d_o = 0.f;
+    if (active) {
+      const float tc = tanhf_(ct);
+      d_o = dh * tc * go * (1.f - go);
+      const float dct = dc + dh * go * (1.f - tc * tc);
+      d_i = dct * gg * gi * (1.f - gi);
+      d_g = dct * gi * (1.f - gg * gg);
+      d_f = dct * cprev * gf * (1.f - gf);
+      dc = dct * gf;
+    }
+    {
+      // two 16-byte publications per gate plane and row: lanes eu = 0 and 8 each store eight units (publish8_bf16)
+      __nv_bfloat16* dp = a.dg + ((size_t)t * Bt + (active ? b : r0)) * 4 * H + j0 + (eu & 8);
+      const bool st_ = active && (eu & 7) == 0;
+      publish8_bf16(dp, d_i, st_);
+      publish8_bf16(dp + (size_t)H, d_f, st_);
+      publish8_bf16(dp + (size_t)2 * H, d_g, st_);
+      publish8_bf16(dp + (size_t)3 * H, d_o, st_);
+    }
+    if (active) {
+      LSTM_TICK(4)
+      LSTM_TICK(5)
+    }
+  }
+  __syncthreads();
+  cluster_barrier();                     // nobody exits while a peer may still read its shared memory
+  if (prof)
+    for (int i = 0; i < 8; ++i) a.dbg[(size_t)blockIdx.x * 16 + 8 + i] = (unsigned long long)pc[i];
+}
+
 #undef LSTM_TICK
 
 // Whether cluster launches of the recurrence are also cooperative.  ncu's kernel replay refuses cooperative cluster
@@ -978,14 +1168,58 @@ int launch_bwd_cluster(const LstmBwdArgs& a, cudaStream_t st) {
   return 0;
 }
 
+// Row-split cluster launch (clusters of 4): returns -1000 when the clusters cannot all be co-resident (caller falls back).
+template <int KS>
+int launch_bwd_rows(const LstmBwdArgs& a, cudaStream_t st) {
+  using SM = BwdRowsSmem<KS>;
+  auto kern = lstm_bwd_rows_kernel<KS>;
+  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::BYTES));
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(a.H / kU);
+  cfg.blockDim = dim3(kThreads);
+  cfg.dynamicSmemBytes = SM::BYTES;
+  cfg.stream = st;
+  cudaLaunchAttribute attrs[2];
+  attrs[0].id = cudaLaunchAttributeClusterDimension;
+  attrs[0].val.clusterDim.x = 4;
+  attrs[0].val.clusterDim.y = 1;
+  attrs[0].val.clusterDim.z = 1;
+  cfg.attrs = attrs;
+  cfg.numAttrs = 1;
+  int nclusters = 0;
+  if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess) {
+    (void)cudaGetLastError();
+    return -1000;
+  }
+  if (nclusters * 4 < a.H / kU) return -1000;
+  attrs[1].id = cudaLaunchAttributeCooperative;   // see launch_bwd_cluster
+  attrs[1].val.cooperative = 1;
+  cfg.numAttrs = coop_launch() ? 2 : 1;
+  LstmBwdArgs args = a;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args);
+  if (e != cudaSuccess) return set_error((int)e, "lstm_bwd row-split launch: %s", cudaGetErrorString(e));
+  return 0;
+}
+
 template <int KS>
 int launch_bwd(const LstmBwdArgs& a, cudaStream_t st) {
   int rc = -1000;
-  // launch form: VQA_B200_LSTM_BWD_CLUSTER = 1 | 2 | 4 forces it (read per call: tests compare the three forms),
-  // otherwise (or 0) clusters of 4, then 2, then the single-CTA kernel, whichever can be co-resident
+  // launch form (both switches are read per call: tests compare the forms):
+  //   VQA_B200_LSTM_BWD_ROWS = 2: the row-split form when Bt >= 2 and it can be co-resident; 1: the unsplit forms.
+  //     Unset: 2, unless VQA_B200_LSTM_BWD_CLUSTER forces an unsplit form.
+  //   VQA_B200_LSTM_BWD_CLUSTER = 1 | 2 | 4 forces the unsplit form; otherwise (or 0) clusters of 4, then 2, then the
+  //     single-CTA kernel, whichever can be co-resident.
   int forced = g_bwd_cluster;
   if (const char* e = getenv("VQA_B200_LSTM_BWD_CLUSTER")) forced = atoi(e);
-  if (forced == 4 || forced == 0) rc = launch_bwd_cluster<KS, 4>(a, st);
+  int rows = g_bwd_rows;
+  if (const char* e = getenv("VQA_B200_LSTM_BWD_ROWS")) {
+    if (strcmp(e, "1") == 0) rows = 1;
+    else if (strcmp(e, "2") == 0) rows = 2;
+    else return set_error(VQA_B200_EINVAL, "VQA_B200_LSTM_BWD_ROWS must be 1 or 2 (got '%s')", e);
+  }
+  if (rows == 0) rows = forced == 0 ? 2 : 1;
+  if (rows == 2 && a.Bt >= 2) rc = launch_bwd_rows<KS>(a, st);
+  if (rc == -1000 && (forced == 4 || forced == 0)) rc = launch_bwd_cluster<KS, 4>(a, st);
   if (rc == -1000 && (forced == 2 || forced == 0)) rc = launch_bwd_cluster<KS, 2>(a, st);
   if (rc == -1000) rc = launch_bwd_plain<KS>(a, st);
   return rc;
@@ -1011,6 +1245,7 @@ extern "C" void vqa_b200_debug_set_lstm(void* device_u64x16, int mode) {
   g_dbg = (unsigned long long*)device_u64x16;
   g_mode = mode & 0xFF;
   g_bwd_cluster = (mode >> 8) & 0xF;   // bits 8..11: force the backward cluster size (1, 2, 4); 0 = auto
+  g_bwd_rows = (mode >> 12) & 0x3;     // bits 12..13: force the backward row split (1 = unsplit, 2 = split); 0 = auto
   g_dbg_ctas = (mode >> 16) & 0xFFFF;  // bits 16..31: CTAs (rows of 16 counters) the buffer holds; 0 = CTA 0 only
   if (g_dbg_ctas < 1) g_dbg_ctas = 1;
 }
