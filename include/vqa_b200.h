@@ -318,7 +318,7 @@ int vqa_b200_kldiv_logsoftmax_bwd(const float* logits, int64_t ldl, const float*
  *   set_mn_desc : override the MN-major shared-memory descriptor strides of every later GEMM (descriptor sweeps);
  *   set_counters: device buffer of 16 uint64 that vqa_b200_gemm fills with pipeline wait-cycle counters of CTA 0/1;
  *   set_lstm    : device buffer of 16 uint64 per CTA for the recurrence kernels' per-phase cycle counters + experiment
- *                 switches (bits 8..11 of `mode` force the backward cluster size; bits 16..31 = the number of CTAs the
+ *                 switches (bits 0..7 of `mode`: 2 skips the MMAs, for timing only; bits 16..31 = the number of CTAs the
  *                 buffer holds, 0 = CTA 0 only; tools/lstm_phase_probe.py). */
 #ifdef VQA_B200_DEBUG
 void vqa_b200_debug_set_mn_desc(uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t kadv_bytes);

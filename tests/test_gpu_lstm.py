@@ -4,6 +4,8 @@ restatement of nn.LSTM (oracle.lstm_batch_first, pinned by the mhbcoatt golden f
 The op computes with bf16 operands and fp32 accumulation / cell state (it is only used in bf16 mode), so the bound is
 north_star's bf16 tolerance: relative L2 error <= 2e-2 on outputs; gradients <= 5e-2 (no singular op in the LSTM).
 """
+import re
+
 import pytest
 import torch
 
@@ -67,33 +69,64 @@ def test_lstm_matches_oracle(Bt, S, E, H, xavier):
 
 
 @pytest.mark.parametrize("Bt,S,E,H", [(5, 6, 24, 128), (20, 9, 40, 256), (32, 17, 64, 512), (26, 48, 300, 1024),
-                                      (1, 200, 300, 1024)])
-def test_lstm_backward_variants_agree(Bt, S, E, H):
-    """The backward recurrence has three launch forms (clusters of 4 / 2 CTAs splitting the contraction, and the
-    single-CTA form used when clusters cannot be co-resident): all must produce the same gradients."""
-    import os
+                                      (1, 200, 300, 1024), (2, 200, 300, 1024)])
+def test_lstm_backward_variants_agree(Bt, S, E, H, monkeypatch):
+    """The recurrence has a cluster form per direction (the default) and a cluster-free pair (VQA_B200_LSTM_CLUSTERS=0,
+    also what runs when the clusters cannot all be co-resident): both must produce the same gradients."""
     from vqa_attention_networks_b200 import ops
     x, params, cot = _case(Bt, S, E, H, 77, True)
     xo = x.double().requires_grad_(True)
     po = [p.double().requires_grad_(True) for p in params]
     (O.lstm_batch_first(xo, *po) * cot.double()).sum().backward()
     grads = {}
-    try:
-        for cl in (1, 2, 4):
-            os.environ["VQA_B200_LSTM_BWD_CLUSTER"] = str(cl)      # read by the library at every launch
-            xg = x.to(DEV).requires_grad_(True)
-            pg = [p.to(DEV).requires_grad_(True) for p in params]
-            out = ops.LstmFn.apply(xg, *pg, ops.WeightCache())
-            (out * cot.to(DEV)).sum().backward()
-            torch.cuda.synchronize()
-            grads[cl] = [xg.grad] + [p.grad for p in pg]
-            for a, b in zip(grads[cl], [xo.grad] + [p.grad for p in po]):
-                assert _rel(a, b) <= 5e-2, (cl, _rel(a, b))
-    finally:
-        os.environ.pop("VQA_B200_LSTM_BWD_CLUSTER", None)
-    for cl in (2, 4):      # same bf16 operands, different summation order only
-        for a, b in zip(grads[cl], grads[1]):
-            assert _rel(a, b) <= 1e-3, (cl, _rel(a, b))
+    for clusters in ("1", "0"):
+        monkeypatch.setenv("VQA_B200_LSTM_CLUSTERS", clusters)      # read by the library at every launch
+        xg = x.to(DEV).requires_grad_(True)
+        pg = [p.to(DEV).requires_grad_(True) for p in params]
+        out = ops.LstmFn.apply(xg, *pg, ops.WeightCache())
+        (out * cot.to(DEV)).sum().backward()
+        torch.cuda.synchronize()
+        grads[clusters] = [xg.grad] + [p.grad for p in pg]
+        for a, b in zip(grads[clusters], [xo.grad] + [p.grad for p in po]):
+            assert _rel(a, b) <= 5e-2, (clusters, _rel(a, b))
+    for a, b in zip(grads["1"], grads["0"]):      # same bf16 operands, different summation order only
+        assert _rel(a, b) <= 1e-3, _rel(a, b)
+
+
+def _launched_lstm_kernels(prof):
+    names = set()
+    for ev in prof.events():
+        m = re.search(r"lstm_\w+_kernel<[^>]*>", ev.name)
+        if m and ev.device_type == torch.autograd.DeviceType.CUDA:
+            names.add(m.group(0).replace(" ", ""))
+    return names
+
+
+@pytest.mark.parametrize("H", [128, 256, 512, 1024])
+@pytest.mark.parametrize("Bt", [1, 26])
+@pytest.mark.parametrize("clusters", [None, "0"])
+def test_lstm_launch_forms(H, Bt, clusters, monkeypatch):
+    """The kernels each form runs: by default the multicast forward in clusters of 4 and the row-split backward, with
+    VQA_B200_LSTM_CLUSTERS=0 the sweep forward and the single-CTA backward.  A silent fallback would make the agreement
+    tests compare a form with itself."""
+    from torch.profiler import ProfilerActivity, profile
+    from vqa_attention_networks_b200 import ops
+    if clusters is None:
+        monkeypatch.delenv("VQA_B200_LSTM_CLUSTERS", raising=False)
+    else:
+        monkeypatch.setenv("VQA_B200_LSTM_CLUSTERS", clusters)
+    x, params, cot = _case(Bt, 4, 24, H, 6, True)
+    xg = x.to(DEV).requires_grad_(True)
+    pg = [p.to(DEV).requires_grad_(True) for p in params]
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        ops.LstmFn.apply(xg, *pg, ops.WeightCache()).backward(cot.to(DEV))
+        torch.cuda.synchronize()
+    ks = H // 128
+    if clusters is None:
+        expected = {"lstm_fwd_kernel<%d,4>" % ks, "lstm_bwd_rows_kernel<%d>" % ks}
+    else:
+        expected = {"lstm_fwd_kernel<%d,1>" % ks, "lstm_bwd_kernel<%d>" % ks}
+    assert _launched_lstm_kernels(prof) == expected
 
 
 def test_lstm_rejects_unsupported_shapes():

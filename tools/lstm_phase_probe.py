@@ -1,7 +1,7 @@
 """Per-phase cycle counters of the recurrence kernels over ALL CTAs, on config 2's shape (S=256 steps over Bt=26 rows,
-300 -> 1024), forward (training form) and backward, for each backward launch form: unsplit clusters of 4 (`rows1`)
-and the row split (`rows2`), forced through the debug hook's mode bits 12..13.  The forward runs in its default form
-(VQA_B200_LSTM_EXCHANGE selects another one).
+300 -> 1024), forward (training form) and backward, for the default cluster forms (`clusters`: multicast forward,
+row-split backward) and the cluster-free pair (`cluster_free`: sweep forward, single-CTA backward), chosen through
+VQA_B200_LSTM_CLUSTERS.
 
 Builds the library with VQA_B200_DEBUG=1 (instrumented kernels + the vqa_b200_debug_set_lstm hook) into a temporary
 copy of the package, so the tree's release library is left alone.  Thread 0 of every CTA accumulates clock64() deltas
@@ -83,15 +83,16 @@ def main():
         dbg = torch.zeros(ncta * 16, dtype=torch.int64, device=dev)
         res = {"card": card(), "shape": {"S": S, "Bt": Bt, "E": E, "H": H}, "unit": "SM cycles (clock64)",
                "note": "thread 0 of every CTA; forward and backward of the last of 5 fwd+bwd calls"}
-        for rows in (1, 2):
-            mode = "rows%d" % rows
-            L.vqa_b200_debug_set_lstm(ctypes_ptr(dbg), (ncta << 16) | (rows << 12))
+        for mode, clusters in (("clusters", "1"), ("cluster_free", "0")):
+            os.environ["VQA_B200_LSTM_CLUSTERS"] = clusters
+            L.vqa_b200_debug_set_lstm(ctypes_ptr(dbg), ncta << 16)
             for _ in range(5):
                 for t in (x, W_ih, W_hh, b):
                     t.grad = None
                 ops.LstmFn.apply(x, W_ih, W_hh, b, b, cache).backward(cot)
             torch.cuda.synchronize()
             L.vqa_b200_debug_set_lstm(None, 0)
+            os.environ.pop("VQA_B200_LSTM_CLUSTERS")
             rows = dbg.view(ncta, 16).cpu().numpy()
             res[mode] = {"forward": summarise(rows[:, :8], FWD_PHASES, S),
                          "backward": summarise(rows[:, 8:], BWD_PHASES, S - 1)}

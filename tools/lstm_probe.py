@@ -4,7 +4,8 @@ ops.LstmFn forward (training and inference form) plus fwd+bwd; the outputs and t
 bit equality against the first form.  S and Bt can be overridden from the environment (S=..., Bt=...).
 
 The A/B subject is one library switch, read at every launch, alternated twice in one process:
-AB="VARIABLE=value1,value2" (default VQA_B200_LSTM_BWD_ROWS=1,2; round 3 used VQA_B200_LSTM_EXCHANGE=sweep,multicast).
+AB="VARIABLE=value1,value2" (default VQA_B200_LSTM_CLUSTERS=0,1: the cluster-free forms against the cluster forms,
+whose backward dg differ from theirs in summation order).
 (Earlier A/B runs with it, round 2: 16-byte publications -45 us forward / -36 us backward; speculative sweeps without the
 canary spin +13 %; one barrier per step with double-buffered partial tiles +13 %; poll backoff +7 %.)
 
@@ -16,7 +17,7 @@ from vqa_attention_networks_b200 import ops
 
 dev = "cuda:0"
 Bt, S, E, H = int(os.environ.get("Bt", 26)), int(os.environ.get("S", 256)), 300, 1024
-var, vals = os.environ.get("AB", "VQA_B200_LSTM_BWD_ROWS=1,2").split("=")
+var, vals = os.environ.get("AB", "VQA_B200_LSTM_CLUSTERS=0,1").split("=")
 vals = vals.split(",")
 g = torch.Generator().manual_seed(0)
 x = torch.tanh(torch.randn(S, Bt, E, generator=g)).permute(1, 0, 2).to(dev).requires_grad_(True)

@@ -4,14 +4,14 @@
 //
 // The recurrence is latency-bound: 2*Bt*4H*H flops per step (0.2 GFLOP at Bt=26, H=1024) behind a
 // grid-wide dependency per step.  The stock path pays two kernel launches per step (a tf32 GEMM and
-// an elementwise cell); here ONE persistent kernel per direction runs the whole sequence (forward: cooperative launch of
-// clusters of 4 CTAs sharing each fetch of h_{t-1} by TMA multicast; backward: clusters of 4 CTAs splitting the
-// contraction, each half of the grid running half of the batch rows; co-residency of the clusters is checked with
-// cudaOccupancyMaxActiveClusters):
-//   * H/8 CTAs (128 at H=1024, one per SM), each owning 8 hidden units = 32 rows of W_hh (forward)
-//     or, in the backward, a share of the contraction for the 64 units of its cluster over half of the rows (see
-//     lstm_bwd_rows_kernel; lstm_bwd_cluster_kernel, 8*CL units over all rows, and the single-CTA lstm_bwd_kernel
-//     are the fallbacks when it does not fit or Bt = 1);
+// an elementwise cell); here ONE persistent kernel per direction runs the whole sequence.  Each direction has a cluster
+// form and a cluster-free form (forward: clusters of 4 CTAs sharing each fetch of h_{t-1} by TMA multicast, or every CTA
+// sweeping it; backward: clusters of 4 CTAs splitting the contraction, each half of the grid running half of the batch
+// rows, or single CTAs).  The cluster forms run unless cudaOccupancyMaxActiveClusters says their clusters cannot all be
+// co-resident, or VQA_B200_LSTM_CLUSTERS=0 asks for the cluster-free pair:
+//   * H/8 CTAs (128 at H=1024, one per SM), each owning 8 hidden units = 32 rows of W_hh (forward and single-CTA
+//     backward), or, in the row-split backward, a share of the contraction for the 64 units of its cluster over half of
+//     the rows (see lstm_bwd_rows_kernel);
 //   * the CTA's slice of W_hh lives in REGISTERS for the whole sequence, already laid out as
 //     mma.sync.m16n8k16 operand fragments (8 warps split the contraction; 64 registers per thread);
 //   * the step-to-step exchange (h_t forward, dgates_t backward; bf16, through L2) carries its own
@@ -117,8 +117,6 @@ __device__ __forceinline__ float tanhf_(float x) { return 1.f - __fdividef(2.f, 
 unsigned long long* g_dbg = nullptr;
 int g_dbg_ctas = 1;
 int g_mode = 0;
-int g_bwd_cluster = 0;      // 0 = auto (4, then 2, then 1), else forced cluster size (debug / A-B timing)
-int g_bwd_rows = 0;         // 0 = auto, 1 = unsplit backward forms, 2 = row-split form (debug / A-B timing)
 enum { MODE_NOMMA = 2 };   // experiment switch: skip the MMAs (results are wrong; timing only)
 
 __device__ __forceinline__ uint32_t cluster_rank() {
@@ -139,8 +137,9 @@ __device__ __forceinline__ void cluster_barrier() {
 // The PTX memory model only PROMISES visibility of the peers' shared-memory writes with release / acquire on the cluster
 // barrier (ADVICE r1); the relaxed form is what the hardware needs today and is 0.16 ms per backward pass faster.
 // -DVQA_B200_LSTM_STRICT_BARRIER (VQA_B200_LSTM_STRICT_BARRIER=1 at build time) selects the guaranteed form, and
-// tests/test_gpu_lstm.py::test_lstm_backward_variants_agree compares the cluster forms against the single-CTA kernel
-// (no cluster exchange at all) at every supported hidden size, so a silent loss of visibility would show as a mismatch.
+// tests/test_gpu_lstm.py::test_lstm_backward_variants_agree compares the row-split backward against the single-CTA kernel
+// (no cluster exchange at all; VQA_B200_LSTM_CLUSTERS=0) at every supported hidden size, so a silent loss of
+// visibility would show as a mismatch.
 __device__ __forceinline__ void step_barrier() {
   __syncthreads();
 #ifdef VQA_B200_LSTM_STRICT_BARRIER
@@ -703,167 +702,18 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_bwd_kernel(const LstmBwdArgs
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Backward recurrence, cluster version.  dh_{t-1}[b, j] = sum_k dgates_t[b, k] W_hh[k, j] contracts over 4H gate columns
-// for only H outputs: with one CTA per 8 units every CTA has to pull ALL of dgates_t (213 KB at Bt=26, H=1024) out of
-// L2 per step.  Here a cluster of CL CTAs owns 8*CL units and splits the contraction CL ways (CTA rank r takes gate
-// columns [r*4H/CL, (r+1)*4H/CL), 53 KB at CL=4 -- the forward's volume), every CTA computes partial sums for all the
-// cluster's units, and the CL partial tiles meet through distributed shared memory: one barrier.cluster per step.
-// ---------------------------------------------------------------------------------------------------------------
-template <int KS, int CL>
-__global__ void __launch_bounds__(kThreads, 1) lstm_bwd_cluster_kernel(const LstmBwdArgs a) {
-  constexpr int KSB = 4 * KS / CL;       // k-steps of one warp's contraction slice (4H / CL / 8 warps / 16)
-  constexpr int PITCH = KSB * 16 + 8;    // (PITCH/2) % 8 == 4 -> conflict-free ldmatrix
-  constexpr int NPROD = 2 * KSB;         // CTAs that produce one warp's slice of dgates
-  constexpr int NU = 8 * CL;             // units of the cluster
-  constexpr int RP = NU + 8;             // pitch of the per-warp partial tiles (floats): 8*b + u is conflict-free
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  __nv_bfloat16* ds = reinterpret_cast<__nv_bfloat16*>(smem_raw);
-  float* red = reinterpret_cast<float*>(smem_raw + (size_t)kWarps * kRows * PITCH * 2);
-  constexpr int PP = NU + 8;             // pitch of the CTA-level partial sums (conflict-free like RP)
-  float* part = red + kWarps * 32 * RP;  // [2][32][PP]: this CTA's partial sums for all units of the cluster
-
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, g = lane >> 2, tg = lane & 3;
-  const int H = a.H, Bt = a.Bt, S = a.S;
-  const uint32_t rank = cluster_rank();
-  const int j0 = blockIdx.x * kU;                    // own units (gate math, dgates output)
-  const int u0 = (blockIdx.x / CL) * NU;             // first unit of the cluster
-  const int kw = (int)rank * (4 * H / CL) + w * KSB * 16;   // first gate column of this warp's contraction slice
-
-  for (int i = tid; i < kWarps * kRows * PITCH / 2; i += kThreads) reinterpret_cast<uint32_t*>(ds)[i] = 0u;
-
-  // W_hh[k, u0 + nt*8 + g] for the warp's k-slice as B fragments (n = unit, k = gate column)
-  uint32_t bfr[KSB][CL][2];
-#pragma unroll
-  for (int ks = 0; ks < KSB; ++ks)
-#pragma unroll
-    for (int nt = 0; nt < CL; ++nt) {
-      const size_t kq = (size_t)kw + ks * 16 + 2 * tg;
-      bfr[ks][nt][0] = ld_w_pair(a.whhT, a.w_layout, (size_t)(u0 + nt * 8 + g), kq, H);
-      bfr[ks][nt][1] = ld_w_pair(a.whhT, a.w_layout, (size_t)(u0 + nt * 8 + g), kq + 8, H);
-    }
-  __syncthreads();
-
-  __nv_bfloat16* dw = ds + (size_t)w * kRows * PITCH;
-  float* redw = red + w * 32 * RP;
-  const int eb = tid >> 3, eu = tid & 7;
-  const bool active = eb < Bt;
-  float dc = 0.f;
-  const bool prof = LSTM_PROF(a);
-  long long pc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tk = 0;
-  const uint32_t dseed = a.drop.thresh16 ? effective_seed(a.drop.seed, a.drop.seed_dev) : 0u;
-
-  // The saved activations of the thread's (row, unit) are pulled into L2 one step ahead (prefetch.global.L2) and read
-  // at the top of their step, long before the gate math needs them.  (Loading them into registers a step ahead made
-  // the compiler park each value with a MOV right behind its load: a full DRAM latency, 15 % of the kernel.)
-  auto prefetch = [&](int t) {
-    const size_t row = (size_t)t * Bt + eb;
-    const size_t o = row * H + j0 + eu;
-    const float* gp = a.gates + row * 4 * H + j0 + eu;
-    prefetch_l2(gp);
-    prefetch_l2(gp + (size_t)H);
-    prefetch_l2(gp + (size_t)2 * H);
-    prefetch_l2(gp + (size_t)3 * H);
-    prefetch_l2(a.c_all + o);
-    prefetch_l2(a.dout + (size_t)t * a.dout_st + (size_t)eb * a.dout_sb + j0 + eu);
-  };
-  if (active && (eu == 0)) prefetch(S - 1);
-  cluster_barrier();                     // every CTA of the cluster is resident before anyone touches remote smem
-
-  for (int t = S - 1; t >= 0; --t) {
-    if (prof) tk = clock64();
-    float gi = 0.f, gf = 0.f, gg = 0.f, go = 0.f, ct = 0.f, cprev = 0.f, dh = 0.f;
-    if (active) {
-      const size_t row = (size_t)t * Bt + eb;
-      const size_t o = row * H + j0 + eu;
-      const float* gp = a.gates + row * 4 * H + j0 + eu;
-      gi = __ldcs(gp);
-      gf = __ldcs(gp + (size_t)H);
-      gg = __ldcs(gp + (size_t)2 * H);
-      go = __ldcs(gp + (size_t)3 * H);
-      ct = __ldcs(a.c_all + o);
-      cprev = t > 0 ? __ldcs(a.c_all + o - (size_t)Bt * H) : 0.f;      // read (and cached) as c_t one step ago
-      dh = drop_out(__ldcs(a.dout + (size_t)t * a.dout_st + (size_t)eb * a.dout_sb + j0 + eu), a.drop, dseed,
-                    (uint32_t)row, (uint32_t)(j0 + eu));
-      if (t > 0 && eu == 0) prefetch(t - 1);         // one lane per 32-byte sector
-    }
-    if (t < S - 1) {                     // uniform over the cluster
-      const __nv_bfloat16* src = a.dg + (size_t)(t + 1) * Bt * 4 * H + kw;
-#pragma unroll 1
-      for (int i = lane; i < NPROD; i += 32) spin_piece(src + (size_t)(Bt - 1) * 4 * H + i * 8);
-      __syncwarp();
-      LSTM_TICK(0)
-      float acc[2][CL][4];
-      const int tries = sweep_mma<KSB, CL>(acc, bfr, dw, src, (size_t)4 * H, Bt, lane, (a.mode & MODE_NOMMA) != 0);
-      LSTM_TICK(1)
-      if (prof) pc[7] += tries;
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-        for (int nt = 0; nt < CL; ++nt) {
-          const int r = mt * 16 + g, uc = nt * 8 + 2 * tg;
-          *reinterpret_cast<float2*>(redw + r * RP + uc) = make_float2(acc[mt][nt][0], acc[mt][nt][1]);
-          *reinterpret_cast<float2*>(redw + (r + 8) * RP + uc) = make_float2(acc[mt][nt][2], acc[mt][nt][3]);
-        }
-      LSTM_TICK(2)
-      __syncthreads();
-      // this CTA's partial sums for all NU units of the cluster (double-buffered by step parity: a remote reader of
-      // step t is done before it arrives at the barrier of step t-1, which precedes our next write to this buffer)
-      float* pbuf = part + (t & 1) * 32 * PP;
-#pragma unroll
-      for (int jj = 0; jj < CL; ++jj) {
-        float sum = 0.f;
-#pragma unroll
-        for (int ww = 0; ww < kWarps; ++ww) sum += red[(ww * 32 + eb) * RP + jj * 8 + eu];
-        pbuf[eb * PP + jj * 8 + eu] = sum;
-      }
-      LSTM_TICK(3)
-      step_barrier();
-      if (active) {
-#pragma unroll
-        for (int rr = 0; rr < CL; ++rr) dh += ld_dsmem_f32(pbuf + eb * PP + (int)rank * 8 + eu, (uint32_t)rr);
-      }
-    }
-    float d_i = 0.f, d_f = 0.f, d_g = 0.f, d_o = 0.f;
-    if (active) {
-      const float tc = tanhf_(ct);
-      d_o = dh * tc * go * (1.f - go);
-      const float dct = dc + dh * go * (1.f - tc * tc);
-      d_i = dct * gg * gi * (1.f - gi);
-      d_g = dct * gi * (1.f - gg * gg);
-      d_f = dct * cprev * gf * (1.f - gf);
-      dc = dct * gf;
-    }
-    {
-      // one 16-byte publication per gate plane and row (see publish8_bf16)
-      __nv_bfloat16* dp = a.dg + ((size_t)t * Bt + (active ? eb : 0)) * 4 * H + j0;
-      const bool st_ = active && eu == 0;
-      publish8_bf16(dp, d_i, st_);
-      publish8_bf16(dp + (size_t)H, d_f, st_);
-      publish8_bf16(dp + (size_t)2 * H, d_g, st_);
-      publish8_bf16(dp + (size_t)3 * H, d_o, st_);
-    }
-    if (active) {
-      LSTM_TICK(4)
-      LSTM_TICK(5)
-    }
-  }
-  __syncthreads();
-  cluster_barrier();                     // nobody exits while a peer may still read its shared memory
-  if (prof)
-    for (int i = 0; i < 8; ++i) a.dbg[(size_t)blockIdx.x * 16 + 8 + i] = (unsigned long long)pc[i];
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// Backward recurrence, row-split version.  A cluster reads Bt * 4H * 2 bytes of dgates_t per step whatever it does
-// inside, since it contracts over all 4H gate columns for the units it owns; total L2 traffic per step is that times
-// the number of clusters, i.e. inversely proportional to the units a cluster owns.  The Bt batch rows are independent
-// recurrences, so the grid is split into two halves that each run half of the rows: cluster (G, h) of 4 CTAs owns the
-// 64 units [64G, 64G + 64) for row half h (rows [0, ceil(Bt/2)) or [ceil(Bt/2), Bt)), which halves the L2 reads and the
-// producers a warp polls against lstm_bwd_cluster_kernel<KS, 4>.  CTA rank r contracts over gate plane r exactly as
-// there (same k-slice per warp, same MMA k order, same warp- and rank-sum order, dh starting from the same masked dout),
-// computes partial sums for the 64 units over one 16-row m-tile, and owns 16 units for the gate math and publication
-// (two 16-byte pieces per gate plane and row).  A row's element is computed the same way whichever m-tile row or n-tile
-// column it sits in, so dgates are bit-identical to the unsplit form.
+// Backward recurrence, row-split cluster version.  dh_{t-1}[b, j] = sum_k dgates_t[b, k] W_hh[k, j] contracts over 4H
+// gate columns for only H outputs: with one CTA per 8 units (lstm_bwd_kernel) every CTA has to pull ALL of dgates_t out
+// of L2 per step.  Here a cluster of 4 CTAs splits the contraction (CTA rank r takes gate plane r), every CTA computes
+// partial sums for all the cluster's units, and the 4 partial tiles meet through distributed shared memory: one
+// barrier.cluster per step.  A cluster reads Bt * 4H * 2 bytes of dgates_t per step whatever it does inside, so total
+// L2 traffic per step is that times the number of clusters, i.e. inversely proportional to the units a cluster owns.
+// The Bt batch rows are independent recurrences, so the grid is split into two halves that each run half of the rows:
+// cluster (G, h) owns the 64 units [64G, 64G + 64) for row half h (rows [0, ceil(Bt/2)) or [ceil(Bt/2), Bt)).  At
+// Bt = 1 the grid is the first half only.  Each CTA computes partial sums for the 64 units over one 16-row m-tile, and
+// owns 16 units for the gate math and publication (two 16-byte pieces per gate plane and row).  A row's element is
+// computed the same way whichever m-tile row or half it sits in, so a row's dgates do not depend on the rows run beside
+// it.
 // Each warp holds B fragments for 8 n-tiles; where they do not all fit in registers (KS = 8) n-tiles 4..7 live in
 // shared memory in lane order.
 // ---------------------------------------------------------------------------------------------------------------
@@ -933,7 +783,9 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_bwd_rows_kernel(const LstmBw
   long long pc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tk = 0;
   const uint32_t dseed = a.drop.thresh16 ? effective_seed(a.drop.seed, a.drop.seed_dev) : 0u;
 
-  // saved activations pulled into L2 one step ahead (see lstm_bwd_cluster_kernel)
+  // The saved activations of the thread's (row, unit) are pulled into L2 one step ahead (prefetch.global.L2) and read
+  // at the top of their step, long before the gate math needs them.  (Loading them into registers a step ahead made
+  // the compiler park each value with a MOV right behind its load: a full DRAM latency, 15 % of the kernel.)
   auto prefetch = [&](int t) {
     const size_t row = (size_t)t * Bt + b;
     const size_t o = row * H + j0 + eu;
@@ -985,8 +837,8 @@ __global__ void __launch_bounds__(kThreads, 1) lstm_bwd_rows_kernel(const LstmBw
       }
       LSTM_TICK(2)
       __syncthreads();
-      // this CTA's partial sums for all 64 units of the cluster, double-buffered by step parity (as in
-      // lstm_bwd_cluster_kernel)
+      // this CTA's partial sums for all 64 units of the cluster (double-buffered by step parity: a remote reader of
+      // step t is done before it arrives at the barrier of step t-1, which precedes our next write to this buffer)
       float* pbuf = part + (t & 1) * 16 * RP;
 #pragma unroll
       for (int jj = 0; jj < 4; ++jj) {
@@ -1045,77 +897,91 @@ bool coop_launch() {
   return coop != 0;
 }
 
-// CL == 1: the sweep form, a cooperative launch.  CL > 1: the multicast form, a cooperative cluster launch; returns
-// -1000 when CL-CTA clusters cannot all be co-resident on this device (caller falls back).
-template <int KS, int CL>
-int launch_fwd(const LstmFwdArgs& a, cudaStream_t st) {
-  using SM = FwdSmem<KS, CL>;
-  auto kern = lstm_fwd_kernel<KS, CL>;
-  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::BYTES));
-  LstmFwdArgs args = a;
-  CUtensorMap hmap;
-  memset(&hmap, 0, sizeof(hmap));
-  if (CL == 1) {
-    void* params[] = {&args, &hmap};
-    VQA_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)kern, dim3(a.H / kU), dim3(kThreads), params, SM::BYTES, st));
-    return 0;
-  }
-  // hb as a [(S+1) * Bt, H] matrix (a batch of one); one box = one column half of a warp's slice over the Bt rows of a step
-  constexpr CUtensorMapSwizzle swz_mode = SM::RB == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                          : SM::RB == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
-  if (int rc = make_tmap(&hmap, a.hb, (uint64_t)a.H, (uint64_t)(a.S + 1) * a.Bt, (uint64_t)a.H, (uint32_t)(SM::RB / 2),
-                         (uint32_t)a.Bt, 1, 0, swz_mode))
-    return rc;
+// VQA_B200_LSTM_CLUSTERS, read at every launch (tests and A/B probes compare the forms in one process): 1, the default,
+// runs the cluster forms; 0 runs the cluster-free pair, the forms a device gets when the clusters cannot all be
+// co-resident.  Returns 1 or 0, or the library error for any other value.
+int clusters_enabled() {
+  const char* e = getenv("VQA_B200_LSTM_CLUSTERS");
+  if (e == nullptr || strcmp(e, "1") == 0) return 1;
+  if (strcmp(e, "0") == 0) return 0;
+  return set_error(VQA_B200_EINVAL, "VQA_B200_LSTM_CLUSTERS must be 0 or 1 (got '%s')", e);
+}
+
+constexpr int kNotCoResident = -1000;   // launch_clusters4 launched nothing: the caller runs its cluster-free form
+
+// Launches `grid` CTAs of `kern` in clusters of 4.  The CTAs wait on each other, so the whole grid must be co-resident:
+// returns kNotCoResident, launching nothing, when cudaOccupancyMaxActiveClusters says the clusters cannot all be.  That
+// query answers for an idle GPU only; under data-parallel training the gradient all-reduce may already hold SMs when
+// this kernel is enqueued, so the launch is COOPERATIVE as well: the grid is only started once all of it fits, instead
+// of resident CTAs spinning on peers that cannot be scheduled.
+template <typename... Params, typename... Args>
+int launch_clusters4(void (*kern)(Params...), int grid, size_t smem, cudaStream_t st, const char* who, Args... args) {
+  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(a.H / kU);
+  cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = SM::BYTES;
+  cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attrs[2];
   attrs[0].id = cudaLaunchAttributeClusterDimension;
-  attrs[0].val.clusterDim.x = CL;
+  attrs[0].val.clusterDim.x = 4;
   attrs[0].val.clusterDim.y = 1;
   attrs[0].val.clusterDim.z = 1;
+  attrs[1].id = cudaLaunchAttributeCooperative;
+  attrs[1].val.cooperative = 1;
   cfg.attrs = attrs;
   cfg.numAttrs = 1;
   int nclusters = 0;
   if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess) {
     (void)cudaGetLastError();
-    return -1000;
+    return kNotCoResident;
   }
-  if (nclusters * CL < a.H / kU) return -1000;
-  attrs[1].id = cudaLaunchAttributeCooperative;   // see launch_bwd_cluster
-  attrs[1].val.cooperative = 1;
+  if (nclusters * 4 < grid) return kNotCoResident;
   cfg.numAttrs = coop_launch() ? 2 : 1;
-  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args, hmap);
-  if (e != cudaSuccess) return set_error((int)e, "lstm_fwd cluster launch: %s", cudaGetErrorString(e));
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+  if (e != cudaSuccess) return set_error((int)e, "%s cluster launch: %s", who, cudaGetErrorString(e));
   return 0;
 }
 
-// Exchange of the forward: VQA_B200_LSTM_EXCHANGE = sweep | multicast (read per call: tests compare the two), multicast
-// by default; VQA_B200_LSTM_FWD_CLUSTER = 2 | 4 forces the cluster size of the multicast form, otherwise (or 0)
-// clusters of 4, then 2, whichever can be co-resident, and the sweep form when neither can.
+// The forward: the multicast form in clusters of 4, else the sweep form (a cooperative launch without clusters).
 template <int KS>
-int launch_fwd_any(const LstmFwdArgs& a, cudaStream_t st) {
-  bool mcast = true;
-  if (const char* e = getenv("VQA_B200_LSTM_EXCHANGE")) {
-    if (strcmp(e, "sweep") == 0) mcast = false;
-    else if (strcmp(e, "multicast") != 0)
-      return set_error(VQA_B200_EINVAL, "VQA_B200_LSTM_EXCHANGE must be sweep or multicast (got '%s')", e);
+int launch_fwd(const LstmFwdArgs& a, cudaStream_t st) {
+  const int clusters = clusters_enabled();
+  if (clusters < 0) return clusters;
+  CUtensorMap hmap;
+  memset(&hmap, 0, sizeof(hmap));
+  if (clusters) {
+    using SM = FwdSmem<KS, 4>;
+    // hb as a [(S+1) * Bt, H] matrix (a batch of one); one box = one column half of a warp's slice over the Bt rows of
+    // a step
+    constexpr CUtensorMapSwizzle swz_mode = SM::RB == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                            : SM::RB == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
+    if (int rc = make_tmap(&hmap, a.hb, (uint64_t)a.H, (uint64_t)(a.S + 1) * a.Bt, (uint64_t)a.H, (uint32_t)(SM::RB / 2),
+                           (uint32_t)a.Bt, 1, 0, swz_mode))
+      return rc;
+    const int rc = launch_clusters4(lstm_fwd_kernel<KS, 4>, a.H / kU, SM::BYTES, st, "lstm_fwd", a, hmap);
+    if (rc != kNotCoResident) return rc;
   }
-  int forced = 0;
-  if (const char* e = getenv("VQA_B200_LSTM_FWD_CLUSTER")) forced = atoi(e);
-  int rc = -1000;
-  if (mcast) {
-    if (forced == 4 || forced == 0) rc = launch_fwd<KS, 4>(a, st);
-    if (rc == -1000 && (forced == 2 || forced == 0)) rc = launch_fwd<KS, 2>(a, st);
-  }
-  if (rc == -1000) rc = launch_fwd<KS, 1>(a, st);
-  return rc;
+  using SM = FwdSmem<KS, 1>;
+  auto kern = lstm_fwd_kernel<KS, 1>;
+  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::BYTES));
+  LstmFwdArgs args = a;
+  void* params[] = {&args, &hmap};
+  VQA_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)kern, dim3(a.H / kU), dim3(kThreads), params, SM::BYTES, st));
+  return 0;
 }
 
+// The backward: the row-split form in clusters of 4, else the single-CTA form (a cooperative launch without clusters).
 template <int KS>
-int launch_bwd_plain(const LstmBwdArgs& a, cudaStream_t st) {
+int launch_bwd(const LstmBwdArgs& a, cudaStream_t st) {
+  const int clusters = clusters_enabled();
+  if (clusters < 0) return clusters;
+  if (clusters) {
+    // two row halves of H/16 CTAs; at Bt = 1 the first only, since the second would hold no rows
+    const int rc = launch_clusters4(lstm_bwd_rows_kernel<KS>, (a.Bt >= 2 ? 2 : 1) * a.H / 16, BwdRowsSmem<KS>::BYTES,
+                                    st, "lstm_bwd", a);
+    if (rc != kNotCoResident) return rc;
+  }
   constexpr int PITCH = KS * 16 + 8;
   const size_t smem = (size_t)kWarps * 2 * kRows * PITCH * 2 + (size_t)kWarps * 32 * 8 * 4;
   VQA_CUDA_CHECK(cudaFuncSetAttribute(lstm_bwd_kernel<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1124,105 +990,6 @@ int launch_bwd_plain(const LstmBwdArgs& a, cudaStream_t st) {
   VQA_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)lstm_bwd_kernel<KS>, dim3(a.H / kU), dim3(kThreads), params,
                                              smem, st));
   return 0;
-}
-
-// Cluster launch: returns -1000 when CL-CTA clusters cannot all be co-resident on this device (caller falls back).
-template <int KS, int CL>
-int launch_bwd_cluster(const LstmBwdArgs& a, cudaStream_t st) {
-  constexpr int KSB = 4 * KS / CL;
-  constexpr int PITCH = KSB * 16 + 8;
-  constexpr int NU = 8 * CL, RP = NU + 8;
-  const size_t smem = (size_t)kWarps * kRows * PITCH * 2 + (size_t)kWarps * 32 * RP * 4 + (size_t)2 * 32 * (NU + 8) * 4;
-  auto kern = lstm_bwd_cluster_kernel<KS, CL>;
-  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(a.H / kU);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attrs[2];
-  attrs[0].id = cudaLaunchAttributeClusterDimension;
-  attrs[0].val.clusterDim.x = CL;
-  attrs[0].val.clusterDim.y = 1;
-  attrs[0].val.clusterDim.z = 1;
-  cfg.attrs = attrs;
-  cfg.numAttrs = 1;
-  int nclusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess) {
-    (void)cudaGetLastError();
-    return -1000;
-  }
-  if (nclusters * CL < a.H / kU) return -1000;
-  // Co-residency of the whole grid is required (CTAs wait on each other).  The occupancy query above answers for an
-  // idle GPU only; under data-parallel training the gradient all-reduce may already hold SMs when this kernel is
-  // enqueued, so the launch is COOPERATIVE as well: the grid is only started once all of it fits, instead of resident
-  // CTAs spinning on peers that cannot be scheduled.
-  if (coop_launch()) {
-    attrs[1].id = cudaLaunchAttributeCooperative;
-    attrs[1].val.cooperative = 1;
-    cfg.numAttrs = 2;
-  }
-  LstmBwdArgs args = a;
-  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args);
-  if (e != cudaSuccess) return set_error((int)e, "lstm_bwd cluster launch: %s", cudaGetErrorString(e));
-  return 0;
-}
-
-// Row-split cluster launch (clusters of 4): returns -1000 when the clusters cannot all be co-resident (caller falls back).
-template <int KS>
-int launch_bwd_rows(const LstmBwdArgs& a, cudaStream_t st) {
-  using SM = BwdRowsSmem<KS>;
-  auto kern = lstm_bwd_rows_kernel<KS>;
-  VQA_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SM::BYTES));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(a.H / kU);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = SM::BYTES;
-  cfg.stream = st;
-  cudaLaunchAttribute attrs[2];
-  attrs[0].id = cudaLaunchAttributeClusterDimension;
-  attrs[0].val.clusterDim.x = 4;
-  attrs[0].val.clusterDim.y = 1;
-  attrs[0].val.clusterDim.z = 1;
-  cfg.attrs = attrs;
-  cfg.numAttrs = 1;
-  int nclusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess) {
-    (void)cudaGetLastError();
-    return -1000;
-  }
-  if (nclusters * 4 < a.H / kU) return -1000;
-  attrs[1].id = cudaLaunchAttributeCooperative;   // see launch_bwd_cluster
-  attrs[1].val.cooperative = 1;
-  cfg.numAttrs = coop_launch() ? 2 : 1;
-  LstmBwdArgs args = a;
-  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args);
-  if (e != cudaSuccess) return set_error((int)e, "lstm_bwd row-split launch: %s", cudaGetErrorString(e));
-  return 0;
-}
-
-template <int KS>
-int launch_bwd(const LstmBwdArgs& a, cudaStream_t st) {
-  int rc = -1000;
-  // launch form (both switches are read per call: tests compare the forms):
-  //   VQA_B200_LSTM_BWD_ROWS = 2: the row-split form when Bt >= 2 and it can be co-resident; 1: the unsplit forms.
-  //     Unset: 2, unless VQA_B200_LSTM_BWD_CLUSTER forces an unsplit form.
-  //   VQA_B200_LSTM_BWD_CLUSTER = 1 | 2 | 4 forces the unsplit form; otherwise (or 0) clusters of 4, then 2, then the
-  //     single-CTA kernel, whichever can be co-resident.
-  int forced = g_bwd_cluster;
-  if (const char* e = getenv("VQA_B200_LSTM_BWD_CLUSTER")) forced = atoi(e);
-  int rows = g_bwd_rows;
-  if (const char* e = getenv("VQA_B200_LSTM_BWD_ROWS")) {
-    if (strcmp(e, "1") == 0) rows = 1;
-    else if (strcmp(e, "2") == 0) rows = 2;
-    else return set_error(VQA_B200_EINVAL, "VQA_B200_LSTM_BWD_ROWS must be 1 or 2 (got '%s')", e);
-  }
-  if (rows == 0) rows = forced == 0 ? 2 : 1;
-  if (rows == 2 && a.Bt >= 2) rc = launch_bwd_rows<KS>(a, st);
-  if (rc == -1000 && (forced == 4 || forced == 0)) rc = launch_bwd_cluster<KS, 4>(a, st);
-  if (rc == -1000 && (forced == 2 || forced == 0)) rc = launch_bwd_cluster<KS, 2>(a, st);
-  if (rc == -1000) rc = launch_bwd_plain<KS>(a, st);
-  return rc;
 }
 
 int check_shape(const char* who, int S, int Bt, int H) {
@@ -1244,8 +1011,6 @@ using namespace vqa;
 extern "C" void vqa_b200_debug_set_lstm(void* device_u64x16, int mode) {
   g_dbg = (unsigned long long*)device_u64x16;
   g_mode = mode & 0xFF;
-  g_bwd_cluster = (mode >> 8) & 0xF;   // bits 8..11: force the backward cluster size (1, 2, 4); 0 = auto
-  g_bwd_rows = (mode >> 12) & 0x3;     // bits 12..13: force the backward row split (1 = unsplit, 2 = split); 0 = auto
   g_dbg_ctas = (mode >> 16) & 0xFFFF;  // bits 16..31: CTAs (rows of 16 counters) the buffer holds; 0 = CTA 0 only
   if (g_dbg_ctas < 1) g_dbg_ctas = 1;
 }
@@ -1382,10 +1147,10 @@ extern "C" int vqa_b200_lstm_fwd(float* gates, const void* whh, float* out, void
                 make_drop(drop_p, seed, seed_dev)};
   cudaStream_t st = (cudaStream_t)stream;
   switch (H / 128) {
-    case 1: return launch_fwd_any<1>(a, st);
-    case 2: return launch_fwd_any<2>(a, st);
-    case 4: return launch_fwd_any<4>(a, st);
-    default: return launch_fwd_any<8>(a, st);
+    case 1: return launch_fwd<1>(a, st);
+    case 2: return launch_fwd<2>(a, st);
+    case 4: return launch_fwd<4>(a, st);
+    default: return launch_fwd<8>(a, st);
   }
 }
 
